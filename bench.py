@@ -1,15 +1,15 @@
 #!/usr/bin/env python
 """bench.py -- phonons traced per second on the BASELINE.json workloads (see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one pass of the propagate path over one batch of phonons: per_gpu phonons on every GPU (weak scaling).
 The default workload is BASELINE.json configs[1], the one the metric is quoted on: the Halfspace near-source model
 (do-halfspace-nearsrc50.sh) at the scripted take-off-angle degree 9, 1.25e8 phonons per GPU and step (its 1e9 phonons over
 the 8 GPUs it is quoted on).  --workload selects any of the five BASELINE configs (halfspace, halfspace_nearsrc50,
-crustpinch, lopnor, spherical), each with its own batch size.  The model is built by the reference's own host code
-(integration/_build/r3d_gpu_main, see radiative3d_b200/reference_host.py).
+crustpinch, lopnor, spherical), each with its own batch size.  The model is built by radiative3d_b200/workload_model.py
+(the workload's geometry as the reference built it, its take-off-angle set, source and scatterer tables at the degree).
 
   value    device-timed (CUDA events on the launching stream, max over ranks): model resident in HBM, K steps plus
            the end-of-run NCCL reduction of the bins (two collectives: the f64 block and the i64 block).
@@ -20,6 +20,11 @@ crustpinch, lopnor, spherical), each with its own batch size.  The model is buil
            `roofline` is the HBM bound (SURVEY 8d bytes), `roofline_issue` the instruction-issue bound the kernel actually
            runs against (warp instructions per loop event from the committed ncu captures, profiles/kernel_counters.json).
   cpu_baseline  the unmodified reference binary (oracle/_ref/r3d_ref_main) on one host core, bounded sample.
+
+--dump-outputs DIR writes what the last timed step computed, as a caller of the path receives it (bins and counters summed
+over ranks), to DIR/energies.npy (f64 [n_seis, n_bins, 5]), DIR/counts.npy and DIR/counters.npy (as f64): that step's
+phonons are traced once more after the timing (phonon i always draws from stream (seed, i)), so two builds run with the
+same arguments can be compared output for output.
 
 --impl reference times the reference's own CPU implementation with all host threads it can use (independent
 processes, the reference's own way of scaling: scripts/do-parallel.sh), on a bounded sample per step.
@@ -187,8 +192,8 @@ def cpu_baseline_port(workload, sample, threads):
     """Fallback when the reference binary did not travel: the C oracle (a port), on `threads` host threads."""
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import oracle_binding as ob
-    from radiative3d_b200 import reference_host
-    m = reference_host.build_model(workload, TOA_DEGREE)
+    from radiative3d_b200 import workload_model
+    m = workload_model.build_model(workload, TOA_DEGREE)
     ob.run(m, 0, min(1000, sample), SEED, nthreads=threads)
     t = time.perf_counter()
     ob.run(m, 0, sample, SEED, nthreads=threads)
@@ -268,7 +273,10 @@ def main():
     ap.add_argument("--per-gpu", type=int, default=None, help="phonons per GPU per step (default: the workload's)")
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's bins and counters as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return reference_arm(args)
     args.warmup = max(args.warmup, 3)
@@ -280,7 +288,7 @@ def main():
     import numpy as np
     import torch
     import torch.distributed as dist
-    from radiative3d_b200 import abi, distributed, engine, reference_host
+    from radiative3d_b200 import abi, distributed, engine, workload_model
     from radiative3d_b200.model import _ARRAYS
 
     rank = int(os.environ.get("RANK", "0"))
@@ -295,8 +303,8 @@ def main():
     if world != args.gpus and rank == 0:
         print(f"bench.py: --gpus {args.gpus} but WORLD_SIZE {world}; using {world}", file=sys.stderr)
 
-    # ---- the model: reference host code builds it, we pin it ------------------------------------------------
-    model = reference_host.build_model(wl, TOA_DEGREE)
+    # ---- the model: built for the workload at the TOA degree, pinned --------------------------------------------
+    model = workload_model.build_model(wl, TOA_DEGREE, device=local)
     keep = []
     for name, _ in _ARRAYS:
         t = torch.from_numpy(getattr(model, name)).pin_memory()
@@ -395,6 +403,18 @@ def main():
                     "note": "the kernel is latency / issue bound, not HBM bound: see roofline_issue"}
         roofline_issue = issue_roofline(wl, kt["events"] / sec, clocks.get("sm_mhz") if clocks else None, kt["ctas"])
 
+    if args.dump_outputs:
+        eng.reset()
+        enqueue(W + K - 1)
+        eng.sync()
+        distributed.all_reduce_blocks(fblk, iblk, k_at)
+        torch.cuda.synchronize()
+        if rank == 0:
+            e, c, k = eng.fetch()
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in (("energies", e), ("counts", c), ("counters", k)):
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a.astype(np.float64))
+
     # ---- e2e: host model in, host bins out, through the C ABI ---------------------------------------------------
     eng.close()
     del fblk, iblk
@@ -466,7 +486,7 @@ def main():
                        "timing": "CUDA events on the launching stream (r3d_sync) + torch events around the reduction, max over ranks",
                        "wall_ms_per_step": 1e3 * wall_s / K,
                        "loop_events_per_second": events_total / dev_s, "events_per_phonon": events_total / total,
-                       "model_built_by": "integration/_build/r3d_gpu_main (reference host code)"},
+                       "model_built_by": "radiative3d_b200/workload_model.py"},
             "clocks": clocks, "gpu_launches": launches,
             "e2e": {"value": per * world / e2e_s, "unit": "phonons/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                     "what": ("r3d_create(pinned host model) + r3d_run + r3d_fetch(pinned host bins) + r3d_destroy, wall clock" if world == 1 else

@@ -1,8 +1,8 @@
 """Parity AT the benchmarked configuration: take-off-angle degree 9 (scripts/do-fundamentals.sh:82), 5 242 880 take-off
 angles, 0.42 GB of CDF tables, 2^23-bucket guide tables - the configuration bench.py measures, not a reduced copy of it.
 
-The models are built on the box by the reference's own host code (integration/_build/r3d_gpu_main, prebuilt where the
-reference checkout exists; radiative3d_b200.reference_host).  Two legs:
+The models are built as bench.py builds them (radiative3d_b200.workload_model, held to the reference's own builds by
+tests/test_workload_model.py).  Two legs:
   * phonon by phonon against the oracle on the same flattened model and the same draw stream (criteria of
     tests/test_gpu_propagate.py: discrete outcome identical for >= 99.5 %, times / path lengths / locations to 1e-8);
   * statistically against runs of the UNMODIFIED reference binary at degree 9 with its own rand() stream
@@ -15,7 +15,7 @@ import numpy as np
 import pytest
 
 import oracle_binding as ob
-from radiative3d_b200 import abi, engine, reference_host
+from radiative3d_b200 import abi, engine, workload_model
 from test_gpu_propagate import compare_finals
 from test_gpu_statistical import compare, gpu_batches, load_stat
 
@@ -27,11 +27,9 @@ _models = {}
 
 
 def model9(cfg):
-    if not os.path.exists(reference_host.GPU_MAIN):
-        pytest.skip("integration/_build/r3d_gpu_main was not built (needs the reference checkout at build time)")
     if cfg not in _models:
         _models.clear()                         # one degree-9 model at a time (up to 4.6 GB of host arrays)
-        _models[cfg] = reference_host.build_model(cfg, 9)
+        _models[cfg] = workload_model.build_model(cfg, 9)
     return _models[cfg]
 
 
