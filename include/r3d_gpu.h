@@ -291,6 +291,49 @@ int r3d_launch_count(r3d_handle *h, uint64_t *n);
 int r3d_set_profiling(r3d_handle *h, int on);
 int r3d_kernel_times(r3d_handle *h, double seconds[3], uint64_t launches[3], uint64_t units[3]);
 
+/* ---- energy snapshots: phonon energy on a voxel grid at chosen lapse times ----------------------------------------------
+ * The energy density E(x, t) of radiative transfer, built in the propagate kernel while each phonon is in registers.
+ *
+ * Contract.  The caller gives K lapse times 0 <= t_0 < t_1 < ... < t_{K-1} <= ttl (K <= R3D_SNAP_MAX_TIMES) and an
+ * axis-aligned grid in model coordinates: origin[3], voxel[3] (> 0), dims[3] (>= 1).
+ *   - Every move of a phonon covers the time interval [t_a, t_b): t_a is its time before Phonon::Move, t_b its time after
+ *     it - the same FP64 value that is the next move's t_a - so the moves of one phonon tile [0, final time) exactly.
+ *   - For every t_k in [t_a, t_b) the phonon makes one record: its position is the point on the move's ray (straight or
+ *     arc) at travel time t_k - t_a from the move's start; its weight is amp^2 = exp(-2 aexp(t_k)), the square of the
+ *     amplitude a seismometer bins; it goes to ray type P = 0 or S = 1.
+ *   - A move makes its records whatever event ends it: scatter, face, hand-over, or loss at a face that does not collect.
+ *     A phonon that times out on an infinite path makes no move and no record; NaN times make none (the comparisons fail).
+ *     So a phonon contributes to snapshot k exactly when its final time is > t_k.
+ *   - The voxel index on each axis is i = floor((x - origin) / voxel), IEEE division.  A record with 0 <= i < dims on all
+ *     three axes goes to that voxel; any other record goes to the snapshot's "outside" cell, so every record is counted.
+ *   - The point at a travel time: straight rays at constant speed (layered cells; shells without velocity gradient) are
+ *     exact, len = dt v.  Curved rays (shell arcs, tetrahedral arcs) take a fixed number of Newton steps on the length
+ *     with Cell::advance's own travel-time formula (radiative3d_b200/csrc/r3d_device.cuh: advance_time).
+ *   - Accumulators per snapshot, voxel (and outside) and ray type: energy (sum of weights, f64) and record count (u64).
+ *     They add up across r3d_run calls, devices and index ranges, like the seismometer bins.
+ * r3d_run launches the kernels with the deposits while snapshots are on; r3d_trace and r3d_trace_events make no snapshot
+ * records.  Snapshots do not change what a phonon does: bins and counters are those of a run without them. */
+#define R3D_SNAP_MAX_TIMES 64
+#define R3D_SNAP_MAX_CELLS (1u << 28)   /* cap on n_times * (dims[0] dims[1] dims[2] + 1) * 2 accumulator cells (4 GB per device) */
+typedef struct r3d_snapshot_desc {
+  uint32_t n_times, reserved;
+  const double *times;     /* [n_times], host memory, borrowed for the call */
+  double origin[3], voxel[3];
+  uint32_t dims[3], reserved2;
+} r3d_snapshot_desc;
+
+/* Synchronise, then give every device of the handle zeroed snapshot accumulators (from the library's private pool),
+ * replacing any earlier grid.  s == NULL or s->n_times == 0 turns snapshots off.  R3D_EINVAL for times that are not
+ * increasing, not finite or outside [0, ttl]; more than R3D_SNAP_MAX_TIMES times; a voxel size that is not finite and
+ * positive; a non-finite origin; a zero dimension; or more than R3D_SNAP_MAX_CELLS accumulator cells.  r3d_reset zeroes
+ * the snapshot accumulators too. */
+int r3d_set_snapshots(r3d_handle *h, const r3d_snapshot_desc *s);
+
+/* Synchronise, sum over the handle's devices, copy out.  Any pointer may be NULL.  energy f64 and count u64:
+ * [n_times][dims[2]][dims[1]][dims[0]][2] (x fastest, last index = ray type); outside_energy, outside_count: [n_times][2].
+ * R3D_EINVAL while snapshots are off. */
+int r3d_fetch_snapshots(r3d_handle *h, double *energy, uint64_t *count, double *outside_energy, uint64_t *outside_count);
+
 /* Parity hook: trace phonons [first, first+n) on device slot 0 WITHOUT touching
  * the accumulators' semantics (bins are still accumulated) and write each
  * phonon's end state to out[n] (host memory). */
@@ -348,6 +391,11 @@ int r3d_test_path_to_boundary(r3d_handle *h, const double *in, uint32_t n, doubl
 /* AdvanceLength (media.cpp:208,442,859): in[i] = {cell,type,x,y,z,theta,phi,len};
  * out as above with face = -1. */
 int r3d_test_advance(r3d_handle *h, const double *in, uint32_t n, double *out);
+
+/* The snapshot deposit's partial advance (see r3d_set_snapshots), with the kernel's device function:
+ * in[i] = {cell, type, x,y,z, theta, phi, dt}: the point reached at travel time dt (0 <= dt < the travel time to the
+ * boundary) along the move to the boundary from that state; out as r3d_test_advance. */
+int r3d_test_advance_time(r3d_handle *h, const double *in, uint32_t n, double *out);
 
 /* Phonon::Transform (phonons.cpp:116-170): in[i] = {theta,phi,pol, rtheta,rphi,rpol};
  * out[i] = {theta,phi,pol}. */

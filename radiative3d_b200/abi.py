@@ -87,6 +87,26 @@ EVENT_DTYPE = np.dtype([
 assert EVENT_DTYPE.itemsize == 96
 
 
+R3D_EINVAL = 1
+R3D_SNAP_MAX_TIMES = 64
+R3D_SNAP_MAX_CELLS = 1 << 28
+
+
+class SnapshotDesc(C.Structure):
+    """struct r3d_snapshot_desc (energy snapshots: lapse times and voxel grid)"""
+    _fields_ = [("n_times", C.c_uint32), ("reserved", C.c_uint32), ("times", _pd),
+                ("origin", C.c_double * 3), ("voxel", C.c_double * 3), ("dims", C.c_uint32 * 3), ("reserved2", C.c_uint32)]
+
+
+def snapshot_desc(times, origin, voxel, dims):
+    """(SnapshotDesc, the float64 times array it points into: keep it alive while the descriptor is used)."""
+    t = np.ascontiguousarray(times, dtype=np.float64).reshape(-1)
+    d = SnapshotDesc(n_times=t.size, times=as_ptr(t, C.c_double))
+    for a in range(3):
+        d.origin[a], d.voxel[a], d.dims[a] = float(origin[a]), float(voxel[a]), int(dims[a])
+    return d, t
+
+
 class ScatterParams(C.Structure):
     """struct r3d_scatter_params (ScatterParams, scatparams.hpp:51-61)"""
     _fields_ = [("nu", C.c_double), ("eps", C.c_double), ("a", C.c_double), ("kappa", C.c_double), ("el", C.c_double), ("gam0", C.c_double)]

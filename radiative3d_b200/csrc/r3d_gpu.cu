@@ -18,6 +18,7 @@
 #include <deque>
 #include <stdlib.h>
 #include <chrono>
+#include <cmath>
 #include "r3d_gpu.h"
 #include "r3d_device.cuh"
 #include "r3d_resident.cuh"
@@ -187,6 +188,26 @@ __global__ void test_path_kernel(const DevModel M, const double *in, uint32_t n,
   o[7] = exp(-t.aexp);
   o[8] = advance_mode ? -1.0 : (double)P.face;
 }
+// in[i] = {cell, type, x,y,z, theta, phi, dt}: the snapshot deposit's partial advance (advance_time) along the move to the
+// boundary from that state
+template <class Cell>
+__global__ void test_advance_time_kernel(const DevModel M, const double *in, uint32_t n, double *out) {
+  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double *x = in + 8 * i;
+  const double *c = M.cell_params + (size_t)(uint32_t)x[0] * M.cell_nparam;
+  const int rt = (int)x[1];
+  const v3 loc = V(x[2], x[3], x[4]), dir = from_thph(x[5], x[6]);
+  typename Cell::Path P;
+  const double len = Cell::path(M, c, rt, loc, dir, P);
+  const Travel seg = Cell::advance(M, c, rt, len, loc, dir, P);
+  const Travel t = advance_time<Cell>(M, c, rt, x[7], loc, dir, P, seg.len, seg.time);
+  double *o = out + 9 * i;
+  o[0] = t.len; o[1] = t.time; o[2] = t.loc.x; o[3] = t.loc.y; o[4] = t.loc.z;
+  if (Cell::curved) angles_of(t.dir, o[5], o[6]); else { o[5] = x[5]; o[6] = x[6]; }
+  o[7] = exp(-t.aexp);
+  o[8] = -1.0;
+}
 __global__ void test_transform_kernel(const double *in, uint32_t n, double *out) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -287,6 +308,10 @@ struct DevState {
   unsigned long long *ibuf = nullptr;
   size_t n_ibuf = 0, n_fbuf = 0;
   const double *raw_theta = nullptr, *raw_phi = nullptr, *raw_spol = nullptr;   // the take-off angles and S->S angles as given (sources of peer copies)
+  // energy snapshots (r3d_set_snapshots): Z.n_times == 0 = off.  Z's three arrays are one pool allocation, snap_mem
+  SnapGrid Z{};
+  void *snap_mem = nullptr;
+  size_t snap_cells = 0;                   // n_times * (n_vox + 1) * 2
 };
 
 }  // namespace
@@ -294,6 +319,7 @@ struct DevState {
 struct r3d_handle {
   std::vector<DevState *> devs;
   uint32_t cell_kind = 0, n_seis = 0, n_bins = 0;
+  double ttl = 0;
   // in-process multi-device handles: the devices' accumulators are summed by a kernel on device slot 0 that reads the
   // other devices' memory over NVLink (peer access), into these staging buffers; one device-to-host copy follows
   bool peer_ok = false;
@@ -348,17 +374,19 @@ int dev_upload(DevState &D, const T **p, const T *host, size_t count) {
   return 0;
 }
 
-typedef void (*propagate_fn)(const DevModel, const Job, uint32_t, uint32_t, unsigned long long *, unsigned long long *);
+typedef void (*propagate_fn)(const DevModel, const Job, uint32_t, uint32_t, unsigned long long *, unsigned long long *, const SnapGrid);
+// snap: the plain kernel with the energy-snapshot deposits (the trace kernels have none)
 template <class Cell>
-propagate_fn pick_propagate_of(bool trace, bool small) {
-  if (small) return trace ? propagate_kernel<Cell, true, true> : propagate_kernel<Cell, false, true>;
-  return trace ? propagate_kernel<Cell, true, false> : propagate_kernel<Cell, false, false>;
+propagate_fn pick_propagate_of(bool trace, bool small, bool snap) {
+  if (snap && !trace) return small ? propagate_kernel<Cell, false, true, true> : propagate_kernel<Cell, false, false, true>;
+  if (small) return trace ? propagate_kernel<Cell, true, true, false> : propagate_kernel<Cell, false, true, false>;
+  return trace ? propagate_kernel<Cell, true, false, false> : propagate_kernel<Cell, false, false, false>;
 }
-propagate_fn pick_propagate(uint32_t kind, bool trace, bool small, bool wide = false) {
+propagate_fn pick_propagate(uint32_t kind, bool trace, bool small, bool wide = false, bool snap = false) {
   switch (kind) {
-    case R3D_CELL_CYLINDER: return wide ? pick_propagate_of<CylinderWide>(trace, small) : pick_propagate_of<Cylinder>(trace, small);
-    case R3D_CELL_SHELL: return pick_propagate_of<Shell>(trace, small);
-    default: return pick_propagate_of<Tetra>(trace, small);
+    case R3D_CELL_CYLINDER: return wide ? pick_propagate_of<CylinderWide>(trace, small, snap) : pick_propagate_of<Cylinder>(trace, small, snap);
+    case R3D_CELL_SHELL: return pick_propagate_of<Shell>(trace, small, snap);
+    default: return pick_propagate_of<Tetra>(trace, small, snap);
   }
 }
 
@@ -644,9 +672,10 @@ int build_device(DevState &D, const r3d_model_desc *d) {
     for (int t = 0; t < 2; t++) D.max_slots[t] = std::max(32u, std::min(D.max_slots[t], (uint32_t)cap / 32 * 32));
   }
   if (D.max_slots[1] < 32) return fail(R3D_EUNSUPPORTED, "shared memory too small for the phonon slots");
-  for (int trace = 0; trace < 2; trace++)
+  for (int variant = 0; variant < 3; variant++)          // plain, trace, plain with snapshots
     for (int wide = 0; wide < (d->cell_kind == R3D_CELL_CYLINDER ? 2 : 1); wide++)
-      CK(cudaFuncSetAttribute(pick_propagate(d->cell_kind, trace != 0, D.table_bytes != 0, wide != 0), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)D.smem_block));
+      CK(cudaFuncSetAttribute(pick_propagate(d->cell_kind, variant == 1, D.table_bytes != 0, wide != 0, variant == 2),
+                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)D.smem_block));
   D.wide_threads = std::min((int)CylinderWide::threads, std::max(32, env_int("R3D_THREADS", CylinderWide::threads) / 32 * 32));
   D.wide = (d->cell_kind == R3D_CELL_CYLINDER) ? env_int("R3D_CYL_WIDE", -1) : 0;      // (-1: decided by the first large job, run_job)
   if (D.wide > 1) D.wide = 1;
@@ -677,6 +706,7 @@ int run_job(DevState &D, const JobReq &jr) {
   cudaEvent_t ev0 = D.ev[0], ev1 = D.ev[1], ek0 = D.ev[2], ek1 = D.ev[3];
   CK(cudaEventRecord(ev0, D.stream));
   const bool trace = jr.finals != nullptr || jr.events != nullptr;
+  const bool snap = !trace && D.Z.n_times > 0;        // (also the pilot launches: they trace part of the job)
   unsigned long long n_launch = 0;
   auto launch = [&](unsigned long long done, unsigned long long n, bool wide) -> int {
     Job J; J.first = jr.first + done; J.n = n; J.seed = jr.seed; J.finals = jr.finals ? jr.finals + done : nullptr;
@@ -690,7 +720,8 @@ int run_job(DevState &D, const JobReq &jr) {
     const int grid = (int)std::min<unsigned long long>((unsigned long long)D.grid, need);
     CK(cudaMemsetAsync(D.M.next_phonon, 0, sizeof(unsigned long long), D.stream));
     if (!n_launch) CK(cudaEventRecord(ek0, D.stream));
-    pick_propagate(D.cell_kind, trace, D.table_bytes != 0, wide)<<<grid, wide ? D.wide_threads : D.threads, smem, D.stream>>>(D.M, J, S, D.table_bytes, D.block_tally, D.block_clock);
+    pick_propagate(D.cell_kind, trace, D.table_bytes != 0, wide, snap)<<<grid, wide ? D.wide_threads : D.threads, smem, D.stream>>>(
+        D.M, J, S, D.table_bytes, D.block_tally, D.block_clock, D.Z);
     D.launches += 1;
     n_launch++;
     return 0;
@@ -788,6 +819,7 @@ void destroy_device(DevState *D) {
     cudaSetDevice(D->device);
     if (D->stream) cudaStreamSynchronize(D->stream);
     for (void *p : D->allocs) cudaFreeAsync(p, D->stream);
+    if (D->snap_mem) cudaFreeAsync(D->snap_mem, D->stream);
     if (D->stream) cudaStreamSynchronize(D->stream);
     for (int i = 0; i < 7; i++) if (D->ev[i]) cudaEventDestroy(D->ev[i]);
     if (D->stream) cudaStreamDestroy(D->stream);
@@ -816,7 +848,7 @@ int r3d_create(const r3d_model_desc *desc, const int *devices, int n_dev, r3d_ha
     return fail(R3D_ENODEV, std::string("no usable CUDA device: ") + (e != cudaSuccess ? cudaGetErrorString(e) : "device count is 0"));
   if (n_dev <= 0) return fail(R3D_EINVAL, "n_dev must be >= 1");
   r3d_handle *h = new r3d_handle();
-  h->cell_kind = desc->cell_kind; h->n_seis = desc->n_seis; h->n_bins = desc->n_bins;
+  h->cell_kind = desc->cell_kind; h->n_seis = desc->n_seis; h->n_bins = desc->n_bins; h->ttl = desc->ttl;
   auto bail = [&](int rc) { std::string keep = g_err; r3d_destroy(h); g_err = keep; return rc; };
   // Several devices: the host arrays cross PCIe ONCE, to device slot 0; the other devices copy the large tables from
   // slot 0's memory (NVLink when the devices are peers, else staged by the driver) and derive their own packed tables
@@ -977,7 +1009,89 @@ int r3d_reset(r3d_handle *h) {
     CK(cudaMemsetAsync(D.M.energies, 0, D.n_fbuf * sizeof(double), D.stream));
     CK(cudaMemsetAsync(D.ibuf, 0, D.n_ibuf * sizeof(unsigned long long), D.stream));
     CK(cudaMemsetAsync(D.block_tally, 0, (size_t)D.grid * R3D_NCOUNTERS * sizeof(unsigned long long), D.stream));
+    if (D.snap_mem) {
+      CK(cudaMemsetAsync(D.Z.energy, 0, D.snap_cells * sizeof(double), D.stream));
+      CK(cudaMemsetAsync(D.Z.count, 0, D.snap_cells * sizeof(unsigned long long), D.stream));
+    }
     CK(cudaStreamSynchronize(D.stream));
+  }
+  return 0;
+}
+
+int r3d_set_snapshots(r3d_handle *h, const r3d_snapshot_desc *s) {
+  DeviceGuard guard;
+  if (!h) return fail(R3D_EINVAL, "null handle");
+  const bool on = s && s->n_times;
+  uint64_t n_vox = 1;
+  if (on) {
+    if (s->n_times > R3D_SNAP_MAX_TIMES) return fail(R3D_EINVAL, "more than R3D_SNAP_MAX_TIMES snapshot times");
+    if (!s->times) return fail(R3D_EINVAL, "null snapshot times");
+    for (uint32_t k = 0; k < s->n_times; k++) {
+      const double t = s->times[k];
+      if (!std::isfinite(t) || t < 0 || t > h->ttl) return fail(R3D_EINVAL, "snapshot times must be finite and within [0, ttl]");
+      if (k && !(t > s->times[k - 1])) return fail(R3D_EINVAL, "snapshot times must be increasing");
+    }
+    for (int a = 0; a < 3; a++) {
+      if (!std::isfinite(s->origin[a])) return fail(R3D_EINVAL, "snapshot grid origin must be finite");
+      if (!std::isfinite(s->voxel[a]) || !(s->voxel[a] > 0)) return fail(R3D_EINVAL, "snapshot voxel sizes must be finite and positive");
+      if (!s->dims[a]) return fail(R3D_EINVAL, "snapshot grid dimensions must be at least 1");
+      n_vox *= s->dims[a];
+      if (n_vox > R3D_SNAP_MAX_CELLS) return fail(R3D_EINVAL, "snapshot grid exceeds R3D_SNAP_MAX_CELLS");
+    }
+    if ((uint64_t)s->n_times * (n_vox + 1) * 2 > R3D_SNAP_MAX_CELLS) return fail(R3D_EINVAL, "snapshot grid exceeds R3D_SNAP_MAX_CELLS");
+  }
+  for (DevState *Dp : h->devs) {
+    DevState &D = *Dp;
+    if (int rc = drain(D)) return rc;
+    CK(cudaSetDevice(D.device));
+    CK(cudaStreamSynchronize(D.stream));
+    if (D.snap_mem) CK(cudaFreeAsync(D.snap_mem, D.stream));
+    D.snap_mem = nullptr; D.snap_cells = 0;
+    D.Z = SnapGrid{};
+    if (!on) continue;
+    const size_t cells = (size_t)s->n_times * (n_vox + 1) * 2;
+    cudaMemPool_t pool;
+    if (int rc = device_pool(D.device, &pool)) return rc;
+    CK(cudaMallocFromPoolAsync(&D.snap_mem, cells * (sizeof(double) + sizeof(unsigned long long)) + R3D_SNAP_MAX_TIMES * sizeof(double),
+                               pool, D.stream));
+    double *t = static_cast<double *>(D.snap_mem);
+    D.Z.times = t;
+    D.Z.energy = t + R3D_SNAP_MAX_TIMES;
+    D.Z.count = reinterpret_cast<unsigned long long *>(D.Z.energy + cells);
+    CK(cudaMemcpyAsync(t, s->times, s->n_times * sizeof(double), cudaMemcpyHostToDevice, D.stream));
+    CK(cudaMemsetAsync(D.Z.energy, 0, cells * (sizeof(double) + sizeof(unsigned long long)), D.stream));
+    for (int a = 0; a < 3; a++) { D.Z.origin[a] = s->origin[a]; D.Z.voxel[a] = s->voxel[a]; D.Z.dims[a] = s->dims[a]; }
+    D.Z.n_vox = (uint32_t)n_vox;
+    D.Z.n_times = s->n_times;
+    D.snap_cells = cells;
+    CK(cudaStreamSynchronize(D.stream));                     // (s->times is borrowed)
+  }
+  return 0;
+}
+
+int r3d_fetch_snapshots(r3d_handle *h, double *energy, uint64_t *count, double *outside_energy, uint64_t *outside_count) {
+  DeviceGuard guard;
+  if (!h) return fail(R3D_EINVAL, "null handle");
+  if (h->devs.empty() || !h->devs[0]->snap_mem) return fail(R3D_EINVAL, "snapshots are off (r3d_set_snapshots)");
+  const size_t cells = h->devs[0]->snap_cells, K = h->devs[0]->Z.n_times, nv = h->devs[0]->Z.n_vox;
+  // the sum over the handle's devices, on the host in device order
+  std::vector<double> e(cells, 0.0), eg(cells);
+  std::vector<unsigned long long> c(cells, 0), cg(cells);
+  for (DevState *Dp : h->devs) {
+    DevState &D = *Dp;
+    if (int rc = drain(D)) return rc;
+    CK(cudaSetDevice(D.device));
+    CK(cudaMemcpyAsync(eg.data(), D.Z.energy, cells * sizeof(double), cudaMemcpyDeviceToHost, D.stream));
+    CK(cudaMemcpyAsync(cg.data(), D.Z.count, cells * sizeof(unsigned long long), cudaMemcpyDeviceToHost, D.stream));
+    CK(cudaStreamSynchronize(D.stream));
+    for (size_t i = 0; i < cells; i++) { e[i] += eg[i]; c[i] += cg[i]; }
+  }
+  for (size_t k = 0; k < K; k++) {
+    const size_t at = k * (nv + 1) * 2;
+    if (energy) memcpy(energy + k * nv * 2, e.data() + at, nv * 2 * sizeof(double));
+    if (count) memcpy(count + k * nv * 2, c.data() + at, nv * 2 * sizeof(uint64_t));
+    if (outside_energy) { outside_energy[2 * k] = e[at + nv * 2]; outside_energy[2 * k + 1] = e[at + nv * 2 + 1]; }
+    if (outside_count) { outside_count[2 * k] = c[at + nv * 2]; outside_count[2 * k + 1] = c[at + nv * 2 + 1]; }
   }
   return 0;
 }
@@ -1140,6 +1254,7 @@ int need_device() {
   if (e != cudaSuccess || count == 0) return fail(R3D_ENODEV, "no usable CUDA device");
   return 0;
 }
+// advance_mode: 0 r3d_test_path_to_boundary, 1 r3d_test_advance, 2 r3d_test_advance_time
 int path_hook(r3d_handle *h, const double *in, uint32_t n, double *out, int advance_mode) {
   DeviceGuard guard;
   if (!h || !in || !out) return fail(R3D_EINVAL, "null argument");
@@ -1151,10 +1266,18 @@ int path_hook(r3d_handle *h, const double *in, uint32_t n, double *out, int adva
   if (int rc = S.up(in, (size_t)n * (advance_mode ? 8 : 7), &din)) return rc;
   if (int rc = S.up((const double *)nullptr, (size_t)n * 9, &dout)) return rc;
   unsigned g = (n + 127) / 128;
-  switch (h->cell_kind) {
-    case R3D_CELL_CYLINDER: test_path_kernel<Cylinder><<<g, 128>>>(D.M, din, n, dout, advance_mode); break;
-    case R3D_CELL_SHELL: test_path_kernel<Shell><<<g, 128>>>(D.M, din, n, dout, advance_mode); break;
-    default: test_path_kernel<Tetra><<<g, 128>>>(D.M, din, n, dout, advance_mode); break;
+  if (advance_mode == 2) {
+    switch (h->cell_kind) {
+      case R3D_CELL_CYLINDER: test_advance_time_kernel<Cylinder><<<g, 128>>>(D.M, din, n, dout); break;
+      case R3D_CELL_SHELL: test_advance_time_kernel<Shell><<<g, 128>>>(D.M, din, n, dout); break;
+      default: test_advance_time_kernel<Tetra><<<g, 128>>>(D.M, din, n, dout); break;
+    }
+  } else {
+    switch (h->cell_kind) {
+      case R3D_CELL_CYLINDER: test_path_kernel<Cylinder><<<g, 128>>>(D.M, din, n, dout, advance_mode); break;
+      case R3D_CELL_SHELL: test_path_kernel<Shell><<<g, 128>>>(D.M, din, n, dout, advance_mode); break;
+      default: test_path_kernel<Tetra><<<g, 128>>>(D.M, din, n, dout, advance_mode); break;
+    }
   }
   CK(cudaGetLastError());
   CK(cudaMemcpy(out, dout, (size_t)n * 9 * sizeof(double), cudaMemcpyDeviceToHost));
@@ -1283,6 +1406,7 @@ int r3d_test_cdf_search(const double *cdf, uint32_t n_cdf, const uint32_t *k, ui
 
 int r3d_test_path_to_boundary(r3d_handle *h, const double *in, uint32_t n, double *out) { return path_hook(h, in, n, out, 0); }
 int r3d_test_advance(r3d_handle *h, const double *in, uint32_t n, double *out) { return path_hook(h, in, n, out, 1); }
+int r3d_test_advance_time(r3d_handle *h, const double *in, uint32_t n, double *out) { return path_hook(h, in, n, out, 2); }
 
 int r3d_test_transform(const double *in, uint32_t n, double *out) {
   return rows_hook([&](double *a, double *b) { test_transform_kernel<<<(n + 127) / 128, 128>>>(a, n, b); }, in, n, 6, 3, out);

@@ -68,6 +68,27 @@ struct Phonon {
   int type;
 };
 
+// ---- energy snapshots (include/r3d_gpu.h r3d_set_snapshots) -----------------------------------------------------------
+// The grids of one device: cell ((k * (n_vox + 1) + v) * 2 + type) holds snapshot k, voxel v (x fastest; v = n_vox is the
+// snapshot's "outside" cell) and ray type.  A kernel parameter of its own, after all others, so that the kernels without
+// snapshots keep their parameter layout.
+struct SnapGrid {
+  const double *times;              // [n_times], increasing, in [0, ttl]
+  double *energy;                   // [n_times][n_vox + 1][2]  sum of amp^2
+  unsigned long long *count;        // [n_times][n_vox + 1][2]  records
+  double origin[3], voxel[3];
+  uint32_t dims[3], n_vox, n_times;
+};
+// One move, as a deposit needs it: everything is what the phonon had in registers when it moved (the move's Path is
+// derived again from the start point, by the same function, only for moves that straddle a snapshot time).
+struct SnapMove {
+  double t_a, t_b, aexp, len, time;  // time before / after Phonon::Move, attenuation exponent before, the move's length and time
+  v3 loc, dir;                       // start point and direction
+  uint32_t cell;
+  int type;
+  bool moved;
+};
+
 // ---- per-thread tallies (dataout.cpp:591-617), flushed once per CTA into its own row.  32-bit per thread (a thread
 // sees a few thousand phonons per launch), 64-bit from the CTA's row onwards. ----------------------------------
 struct Tally {
@@ -440,8 +461,8 @@ R3D_DEV void route(const Slots<TRACE> &A, Ctl &C, int nxt, int out, uint32_t s) 
 // =====================================================================================================
 // phase 1a: one Propagate-loop iteration up to the event's classification (phonons.cpp:542-623)
 // =====================================================================================================
-template <class Cell, bool TRACE, class TabT>
-R3D_DEV int advance_one(const DevModel &M, const Job &J, const Slots<TRACE> &A, const TabT &tab, uint32_t s, Tally &T) {
+template <class Cell, bool TRACE, bool SNAP, class TabT>
+R3D_DEV int advance_one(const DevModel &M, const Job &J, const Slots<TRACE> &A, const TabT &tab, uint32_t s, Tally &T, SnapMove &D) {
   Phonon p;
   const Clock4 ck = A.clock(s);
   const double2 lxy = A.lxy(s), lzdz = A.lzdz(s), dxy = A.dxy(s);
@@ -491,9 +512,14 @@ R3D_DEV int advance_one(const DevModel &M, const Job &J, const Slots<TRACE> &A, 
     else {
       const bool scatter = scatlen < edgelen;
       const Travel tr = Cell::advance(M, c, p.type, scatter ? scatlen : edgelen, p.loc, p.dir, P);
+      if (SNAP) {
+        D.t_a = p.time; D.aexp = p.aexp; D.len = tr.len; D.time = tr.time;
+        D.loc = p.loc; D.dir = p.dir; D.cell = p.cell; D.type = p.type; D.moved = true;
+      }
       // Phonon::Move (phonons.cpp:62-70)
       p.pathlen += tr.len; p.time += tr.time; p.recent += tr.time;
       p.loc = tr.loc; p.aexp += tr.aexp; p.moves += 1;
+      if (SNAP) D.t_b = p.time;
       if (Cell::curved) {            // the ray turned: the polarisation ANGLE is what the reference carries along
         const double2 sxy = A.sxy(s);
         p.s1 = carry_pol(p.dir, V(sxy.x, sxy.y, A.sz(s)), tr.dir);
@@ -878,12 +904,76 @@ R3D_DEV void bend_one(const DevModel &M, const Job &J, const Slots<TRACE> &A, co
 }
 
 // =====================================================================================================
+// phase 1b (SNAP kernels): the energy-snapshot records of the moves of one advance chunk.  A move over [t_a, t_b) makes
+// one record for every snapshot time t_k in [t_a, t_b): the point at travel time t_k - t_a along the move (advance_time),
+// weight amp^2 = exp(-2 aexp(t_k)), into the voxel floor((x - origin) / voxel) on each axis or the snapshot's outside cell.
+// At early snapshot times most records of a warp fall into the same few voxels around the source, so the warp aggregates:
+// lanes with the same (snapshot, voxel, type) find each other with one match.any, sum their weights in five shuffle rounds
+// (pointer jumping along the lanes of the key), and the lowest lane adds the sum and the record count with one atomic each.
+// A move can straddle several snapshot times: the warp repeats until no lane has a record left.  All 32 lanes call this.
+// =====================================================================================================
+template <class Cell, class TabT>
+R3D_DEV void snap_deposit(const DevModel &M, const SnapGrid &Z, const TabT &tab, const SnapMove &D) {
+  const unsigned lane = threadIdx.x & 31u;
+  uint32_t k = Z.n_times;
+  if (D.moved) {                                // first k with t_k >= t_a (none for a NaN t_a)
+    uint32_t lo = 0, hi = Z.n_times;
+    while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (__ldg(Z.times + mid) < D.t_a) lo = mid + 1; else hi = mid; }
+    k = lo;
+  }
+  double tk = 0.0;
+  if (k < Z.n_times) tk = __ldg(Z.times + k);
+  bool pending = k < Z.n_times && D.t_a <= tk && tk < D.t_b;            // (false for NaN times)
+  if (!__any_sync(R3D_FULL, pending)) return;
+  typename Cell::Path P;
+  const double *c = nullptr;
+  if (pending) { c = tab.cell(M, D.cell); Cell::path(M, c, D.type, D.loc, D.dir, P); }
+  do {
+    uint32_t key = 0xffffffffu;
+    double w = 0.0;
+    if (pending) {
+      const Travel tr = advance_time<Cell>(M, c, D.type, tk - D.t_a, D.loc, D.dir, P, D.len, D.time);
+      w = exp(-2.0 * (D.aexp + tr.aexp));
+      const double x[3] = {tr.loc.x, tr.loc.y, tr.loc.z};
+      uint32_t v = 0, stride = 1;
+      bool inside = true;
+#pragma unroll
+      for (int a = 0; a < 3; a++) {
+        const double f = floor((x[a] - Z.origin[a]) / Z.voxel[a]);            // IEEE division, as the contract states
+        inside = inside && f >= 0.0 && f < (double)Z.dims[a];
+        if (inside) v += (uint32_t)f * stride;
+        stride *= Z.dims[a];
+      }
+      key = ((k * (Z.n_vox + 1u) + (inside ? v : Z.n_vox)) << 1) | (uint32_t)D.type;
+    }
+    const unsigned peers = __match_any_sync(R3D_FULL, key);
+    const unsigned above = peers & ~((2u << lane) - 1u);     // (lane 31: 2u << 31 wraps to 0, nothing above)
+    int nxt = above ? __ffs(above) - 1 : -1;                  // next lane of the same key
+    for (int r = 0; r < 5; r++) {                             // after round r each lane holds the sum of 2^(r+1) lanes of its key
+      const int src = nxt >= 0 ? nxt : (int)lane;
+      const double x = __shfl_sync(R3D_FULL, w, src);
+      const int nn = __shfl_sync(R3D_FULL, nxt, src);
+      if (nxt >= 0) { w += x; nxt = nn; }
+    }
+    if (pending && (int)lane == __ffs(peers) - 1) {
+      atomicAdd(Z.energy + key, w);
+      atomicAdd(Z.count + key, (unsigned long long)__popc(peers));
+    }
+    if (pending) {
+      k++;
+      if (k < Z.n_times) tk = __ldg(Z.times + k);
+      pending = k < Z.n_times && tk < D.t_b;
+    }
+  } while (__any_sync(R3D_FULL, pending));
+}
+
+// =====================================================================================================
 // the kernel: persistent CTAs, S slots each
 // =====================================================================================================
-template <class Cell, bool TRACE, bool SMALL>
+template <class Cell, bool TRACE, bool SMALL, bool SNAP>
 __global__ void __launch_bounds__(Cell::threads, 1)
 propagate_kernel(const DevModel M, const Job J, uint32_t S, uint32_t table_bytes, unsigned long long *block_tally,
-                 unsigned long long *block_clock) {
+                 unsigned long long *block_clock, const SnapGrid Z) {
   __shared__ unsigned long long tally_sm[R3D_NT / 32][R3D_NCOUNTERS];
   __shared__ Ctl C;
   Slots<TRACE> A; A.S = S; A.table_bytes = table_bytes;
@@ -939,7 +1029,10 @@ propagate_kernel(const DevModel M, const Job J, uint32_t S, uint32_t table_bytes
         const long long tc = clock64();
 #endif
         const uint32_t j = c * 32u + lane;
-        if (j < nA) { s = q[j]; out = advance_one<Cell, TRACE>(M, J, A, tab, s, T); }
+        SnapMove D;
+        D.moved = false;
+        if (j < nA) { s = q[j]; out = advance_one<Cell, TRACE, SNAP>(M, J, A, tab, s, T, D); }
+        if (SNAP) snap_deposit<Cell>(M, Z, tab, D);
         if (out == OUT_FREE) out = OUT_SRC;                     // list B: wants a new phonon in this iteration's phase 2
         route<TRACE>(A, C, nxt, out, s);
 #if R3D_CHUNK_CLOCKS

@@ -22,7 +22,7 @@ _lib = None
 EXPORTS = [
     "r3d_create", "r3d_run", "r3d_sync", "r3d_fetch", "r3d_reset", "r3d_device_accumulators", "r3d_device_accumulator_blocks", "r3d_stream",
     "r3d_launch_count", "r3d_trace", "r3d_trace_events", "r3d_build_scatterer_tables", "r3d_toa_create", "r3d_scatterer_g_values", "r3d_toa_destroy", "r3d_set_profiling", "r3d_kernel_times", "r3d_test_cdf_search", "r3d_test_path_to_boundary", "r3d_test_advance",
-    "r3d_test_transform", "r3d_test_rtcoef", "r3d_test_catch", "r3d_test_arith", "r3d_test_pathlog", "r3d_destroy", "r3d_last_error", "r3d_abi_version",
+    "r3d_test_advance_time", "r3d_set_snapshots", "r3d_fetch_snapshots", "r3d_test_transform", "r3d_test_rtcoef", "r3d_test_catch", "r3d_test_arith", "r3d_test_pathlog", "r3d_destroy", "r3d_last_error", "r3d_abi_version",
 ]
 
 
@@ -63,6 +63,9 @@ def load_library(path=None):
     L.r3d_test_cdf_search.argtypes = [pd, C.c_uint32, pu32, C.c_uint32, pu32, C.c_int]
     L.r3d_test_path_to_boundary.argtypes = [vp, pd, C.c_uint32, pd]
     L.r3d_test_advance.argtypes = [vp, pd, C.c_uint32, pd]
+    L.r3d_test_advance_time.argtypes = [vp, pd, C.c_uint32, pd]
+    L.r3d_set_snapshots.argtypes = [vp, C.POINTER(abi.SnapshotDesc)]
+    L.r3d_fetch_snapshots.argtypes = [vp, pd, pu64, pd, pu64]
     L.r3d_test_transform.argtypes = [pd, C.c_uint32, pd]
     L.r3d_test_rtcoef.argtypes = [pd, C.c_uint32, pd]
     L.r3d_test_arith.argtypes = [pd, C.c_uint32, pd]
@@ -184,6 +187,32 @@ class Engine:
             raise R3DError(abi.R3D_EINVAL if hasattr(abi, "R3D_EINVAL") else 1, f"{n.value} events occurred, room for {cap}")
         return out[:n.value]
 
+    # -- energy snapshots (include/r3d_gpu.h r3d_set_snapshots) --
+    def set_snapshots(self, times, origin=None, voxel=None, dims=None):
+        """Record phonon energy at the lapse `times` (increasing, in [0, ttl], at most 64) on the voxel grid `origin`,
+        `voxel` (sizes), `dims` (nx, ny, nz), in model coordinates, during the following runs; zeroed accumulators.
+        `times` None or empty turns snapshots off."""
+        if times is None or len(times) == 0:
+            _ck(self._L, self._L.r3d_set_snapshots(self._h, None))
+            self._snap = None
+            return
+        d, t = abi.snapshot_desc(times, origin, voxel, dims)
+        _ck(self._L, self._L.r3d_set_snapshots(self._h, C.byref(d)))
+        self._snap = (t.size, tuple(int(x) for x in dims))
+
+    def fetch_snapshots(self):
+        """(energy[K, nz, ny, nx, 2] f64, count[K, nz, ny, nx, 2] u64, outside_energy[K, 2], outside_count[K, 2]) summed
+        over the devices; the last axis is the ray type (P, S)."""
+        if getattr(self, "_snap", None) is None:
+            raise R3DError(abi.R3D_EINVAL, "snapshots are off (set_snapshots)")
+        k, (nx, ny, nz) = self._snap
+        e = np.zeros((k, nz, ny, nx, 2))
+        c = np.zeros((k, nz, ny, nx, 2), dtype=np.uint64)
+        oe = np.zeros((k, 2))
+        oc = np.zeros((k, 2), dtype=np.uint64)
+        _ck(self._L, self._L.r3d_fetch_snapshots(self._h, _pd(e), abi.as_ptr(c, C.c_uint64), _pd(oe), abi.as_ptr(oc, C.c_uint64)))
+        return e, c, oe, oc
+
     @property
     def launch_count(self):
         n = C.c_uint64()
@@ -239,6 +268,11 @@ class Engine:
 
     def advance(self, x):
         return self._rows(self._L.r3d_test_advance, 8, 9, x)
+
+    def advance_time(self, x):
+        """rows {cell, type, x, y, z, theta, phi, dt} -> the snapshot deposit's point at travel time dt along the move to
+        the boundary, as rows of advance()"""
+        return self._rows(self._L.r3d_test_advance_time, 8, 9, x)
 
 
 def _free_rows(name, win, wout, x, *pre):
