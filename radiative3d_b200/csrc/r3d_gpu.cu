@@ -1166,6 +1166,8 @@ int r3d_kernel_times(r3d_handle *h, double seconds[3], uint64_t launches[3], uin
     for (int i = 0; i < 4; i++)
       fprintf(stderr, "r3d chunks: %-8s %10llu chunks, %8.0f cycles each, %5.1f %% of warp time\n", nm[i], k[7 + i],
               k[7 + i] ? (double)k[3 + i] / (double)k[7 + i] : 0.0, 100.0 * (double)k[3 + i] / tot);
+    fprintf(stderr, "r3d chunks: face_collect %8.0f cycles per face chunk, %5.1f %% of face-chunk time (the rest: face_one)\n",
+            k[9] ? (double)k[12] / (double)k[9] : 0.0, k[5] ? 100.0 * (double)k[12] / (double)k[5] : 0.0);
     fprintf(stderr, "r3d chunks: waiting at barriers / for work: %5.1f %% of warp time; phase 1 %.0f, phase 2 %.0f cycles per iteration\n",
             100.0 * (double)k[11] / tot, (double)c1 / (double)std::max(1ull, k[2]), (double)c2 / (double)std::max(1ull, k[2]));
   }

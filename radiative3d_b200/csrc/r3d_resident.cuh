@@ -230,8 +230,9 @@ R3D_DEV double neg_log_unit(const double2 *tab, double r) {
 // S faces, bends
 // per-CTA clocks written at the end of a launch: [0] cycles in phase 1, [1] cycles in phase 2, [2] iterations,
 // [3..6] warp-cycles inside advance / bend / face / draw chunks, [7..10] number of such chunks, [11] warp-cycles
-// spent outside chunks (barriers, waiting for the last chunk of a phase)
-#define R3D_NCLOCKS 12
+// spent outside chunks (barriers, waiting for the last chunk of a phase), [12] of the face chunks' warp-cycles, those in
+// seismometer collection (collect_warp)
+#define R3D_NCLOCKS 13
 struct Ctl {
   unsigned long long t_kind[4], t_idle;
   uint32_t n_kind[4];
@@ -240,6 +241,7 @@ struct Ctl {
   uint32_t cnt[9];
   unsigned long long t_phase[2];    // clock cycles spent in phase 1 / phase 2 (thread 0's view)
   uint32_t iterations;
+  unsigned long long t_collect;     // warp-cycles of the face chunks spent in collect_warp
 };
 enum { CNT_SCAT = 4, CNT_SRC, CNT_FP, CNT_FS, CNT_BEND };
 
@@ -762,14 +764,17 @@ R3D_DEV void draw_batch(const DevModel &M, const Job &J, const Slots<TRACE> &A, 
 // phase 2b, first half: DataReporter::ReportPhononCollected (dataout.cpp:545-568) + Seismometer::CatchPhonon (dataout.cpp:
 // 103-216) for the slots of one face chunk - as a WARP.  Every seismometer is pass-through (dataout.cpp:50), so all that
 // contain the arrival point must bin it; candidates come from the uniform grid over the seismometers' bounding spheres.
-// Few lanes of a chunk arrive at a collecting face, and each has a list of 10-20 candidates: lane by lane (even with the
-// lanes meeting at their n-th candidate) the scan ran at 1.4 of 32 lanes and the exact test at 1.3-2, 6.8 % of the warp
-// instructions and 10 % of the stall samples of the whole-Earth model.  Here the warp takes the arrivals one at a time
-// and spreads each one's candidates over its lanes: the arrival's state is read from its slot in shared memory by all
-// lanes (one broadcast read per field), 32 candidates get the sphere pre-test at once, and the lanes whose candidate passed
-// run the exact test and the bin update together.  The bins go straight to L2 as reductions (red.global.add.f64 / .u64:
-// 5.3e7 sectors in 124 ms on that model = 0.009 % of the L1-to-L2 write throughput, profiles/r2_histogram.md), so there is
-// nothing for an aggregation step in shared memory to win; catches per (seismometer, bin) are independent arrivals.
+// Few lanes of a chunk arrive at a collecting face, each with a short list of candidates (3 on the halfspace models,
+// 10-20 on the whole-Earth model): lane by lane the scan ran at 1.4 of 32 lanes, and one warp pass per arrival (its
+// candidates spread over the lanes) made the passes a serial chain as long as the number of arrivals with candidates -
+// 5-7 per chunk, each at a few active lanes.  So the warp enumerates the chunk's (arrival, candidate) pairs instead: a warp
+// scan of the candidate counts numbers them, and pass b gives pair 32 b + lane to the lane, which finds the arrival that
+// owns it by a binary search over the scanned counts (five shuffles) and reads that arrival's state from its slot in
+// shared memory.  ceil(pairs / 32) passes: one for a typical chunk of the halfspace models.  Every pair gets the same
+// sphere pre-test and, if it passes, the same exact test and bin update as before, on the same operands.  The bins go
+// straight to L2 as reductions (red.global.add.f64 / .u64: 5.3e7 sectors in 124 ms on the whole-Earth model = 0.009 % of
+// the L1-to-L2 write throughput, profiles/r2_histogram.md), so there is nothing for an aggregation step in shared memory
+// to win; catches per (seismometer, bin) are independent arrivals.
 // All 32 lanes call this; `have` = the lane holds a slot of the chunk.
 // =====================================================================================================
 template <class Cell, bool TRACE, class TabT>
@@ -793,44 +798,56 @@ R3D_DEV void collect_warp(const DevModel &M, const Slots<TRACE> &A, const TabT &
       }
     }
   }
-  unsigned pending = __ballot_sync(R3D_FULL, i0 < i1);
-  while (pending) {
-    const int src = __ffs(pending) - 1;
-    pending &= pending - 1u;
-    const uint32_t ss = __shfl_sync(R3D_FULL, s, src), b0 = __shfl_sync(R3D_FULL, i0, src), b1 = __shfl_sync(R3D_FULL, i1, src);
-    // the arrival (same addresses in every lane: broadcast reads)
-    const double t_alive = A.time(ss), aexp = A.aexp(ss);
-    const double2 lxy = A.lxy(ss), lzdz = A.lzdz(ss), dxy = A.dxy(ss), sxy = A.sxy(ss);
-    const uint4 meta = A.meta(ss);
-    const v3 loc = V(lxy.x, lxy.y, lzdz.x), dir = V(dxy.x, dxy.y, lzdz.y);
-    const int type = (int)meta.w;
-    const v3 dopm = (type == R3D_RAY_P) ? dir : V(sxy.x, sxy.y, A.sz(ss));     // Phonon::DirectionOfMotion (phonons.cpp:201-211)
-    uint32_t caught = 0;
-    for (uint32_t base = b0; base < b1; base += 32u) {
-      const uint32_t j = base + lane;
-      if (j < b1) {
-        const uint32_t k2 = __ldg(M.grid_items + j);
-        const double2 qa = __ldg(reinterpret_cast<const double2 *>(M.seis_sphere + k2));
-        const double2 qb = __ldg(reinterpret_cast<const double2 *>(M.seis_sphere + k2) + 1);
-        const double ddx = qa.x - loc.x, ddy = qa.y - loc.y, ddz = qb.x - loc.z;
-        if (ddx * ddx + ddy * ddy + ddz * ddz <= qb.y) {            // may be within the gather radius: the exact CatchPhonon test
-          const double vel = Cell::veloc(tab.cell(M, meta.y), type, loc);
-          uint32_t bin; double e[4];
-          if (seis_catch(M.seis + (size_t)k2 * R3D_SEIS_NPARAM, M.bin_dt, M.n_bins, t_alive, loc, dir, dopm, type, exp(-aexp), vel, bin, e)) {
-            const size_t bb = (size_t)k2 * M.n_bins + bin;
-            atomicAdd(M.energies + bb * 5 + 0, e[0]);
-            atomicAdd(M.energies + bb * 5 + 1, e[1]);
-            atomicAdd(M.energies + bb * 5 + 2, e[2]);
-            atomicAdd(M.energies + bb * 5 + 3 + type, e[3]);
-            atomicAdd(M.counts + bb * 2 + type, 1ull);
-            caught++;
-          }
+  // end = this lane's pairs and those of the lanes below it (inclusive scan); pair p belongs to the lowest lane with end > p
+  const uint32_t n = i1 - i0;
+  uint32_t end = n;
+#pragma unroll
+  for (unsigned o = 1; o < 32u; o <<= 1) {
+    const uint32_t x = __shfl_up_sync(R3D_FULL, end, o);
+    if (lane >= o) end += x;
+  }
+  const uint32_t total = __shfl_sync(R3D_FULL, end, 31);
+  const uint32_t off = i0 - (end - n);                 // candidate of pair p = grid_items[off + p] (mod 2^32)
+  uint32_t caught = 0;
+  for (uint32_t base = 0; base < total; base += 32u) {
+    const uint32_t p = base + lane;
+    uint32_t owner = 0;                                 // lanes below the owner: those with end <= p
+#pragma unroll
+    for (uint32_t step = 16; step > 0; step >>= 1) {
+      if (__shfl_sync(R3D_FULL, end, owner + step - 1u) <= p) owner += step;
+    }
+    const uint32_t ss = __shfl_sync(R3D_FULL, s, owner), j = __shfl_sync(R3D_FULL, off, owner) + p;
+    if (p < total) {
+      const uint32_t k2 = __ldg(M.grid_items + j);
+      const double2 qa = __ldg(reinterpret_cast<const double2 *>(M.seis_sphere + k2));
+      const double2 qb = __ldg(reinterpret_cast<const double2 *>(M.seis_sphere + k2) + 1);
+      const double2 lxy = A.lxy(ss), lzdz = A.lzdz(ss);
+      const v3 loc = V(lxy.x, lxy.y, lzdz.x);
+      const double ddx = qa.x - loc.x, ddy = qa.y - loc.y, ddz = qb.x - loc.z;
+      if (ddx * ddx + ddy * ddy + ddz * ddz <= qb.y) {            // may be within the gather radius: the exact CatchPhonon test
+        const double t_alive = A.time(ss), aexp = A.aexp(ss);
+        const double2 dxy = A.dxy(ss);
+        const uint4 meta = A.meta(ss);
+        const v3 dir = V(dxy.x, dxy.y, lzdz.y);
+        const int type = (int)meta.w;
+        v3 dopm = dir;                                            // Phonon::DirectionOfMotion (phonons.cpp:201-211)
+        if (type != R3D_RAY_P) { const double2 sxy = A.sxy(ss); dopm = V(sxy.x, sxy.y, A.sz(ss)); }
+        const double vel = Cell::veloc(tab.cell(M, meta.y), type, loc);
+        uint32_t bin; double e[4];
+        if (seis_catch(M.seis + (size_t)k2 * R3D_SEIS_NPARAM, M.bin_dt, M.n_bins, t_alive, loc, dir, dopm, type, exp(-aexp), vel, bin, e)) {
+          const size_t bb = (size_t)k2 * M.n_bins + bin;
+          atomicAdd(M.energies + bb * 5 + 0, e[0]);
+          atomicAdd(M.energies + bb * 5 + 1, e[1]);
+          atomicAdd(M.energies + bb * 5 + 2, e[2]);
+          atomicAdd(M.energies + bb * 5 + 3 + type, e[3]);
+          atomicAdd(M.counts + bb * 2 + type, 1ull);
+          caught++;
+          if (TRACE) atomicAdd(&A.tr(0, ss), 1u);                 // catches are rare: one shared atomic each
         }
       }
     }
-    T.v[R3D_CNT_CATCHES] += caught;                    // (a tally is summed over the threads at the end: whose it is does not matter)
-    if (TRACE && caught) atomicAdd(&A.tr(0, ss), caught);
   }
+  T.v[R3D_CNT_CATCHES] += caught;                      // (a tally is summed over the threads at the end: whose it is does not matter)
 }
 
 // =====================================================================================================
@@ -987,7 +1004,7 @@ propagate_kernel(const DevModel M, const Job J, uint32_t S, uint32_t table_bytes
     C.cnt[OUT_FREE] = S;
     C.exhausted = 0; C.done = 0; C.grant_a = 0; C.grant_b = 0; C.t_phase[0] = 0; C.t_phase[1] = 0; C.iterations = 0;
     for (int k = 0; k < 4; k++) { C.t_kind[k] = 0; C.n_kind[k] = 0; }
-    C.t_idle = 0;
+    C.t_idle = 0; C.t_collect = 0;
   }
   const unsigned lane = threadIdx.x & 31u;
   Tally T; T.clear();
@@ -1094,7 +1111,13 @@ propagate_kernel(const DevModel M, const Job J, uint32_t S, uint32_t table_bytes
           uint32_t s = 0;
           const bool have = j < count;
           if (have) s = qf[from_back ? S - 1u - j : j];
+#if R3D_CHUNK_CLOCKS
+          const long long tcc = clock64();
+#endif
           collect_warp<Cell, TRACE>(M, A, tab, have, s, T);
+#if R3D_CHUNK_CLOCKS
+          if (lane == 0) atomicAdd(&C.t_collect, (unsigned long long)(clock64() - tcc));
+#endif
           if (have) out = face_one<Cell, TRACE>(M, J, A, tab, s, T);
           route<TRACE>(A, C, nxt, out, s);
         } else {
@@ -1139,7 +1162,7 @@ propagate_kernel(const DevModel M, const Job J, uint32_t S, uint32_t table_bytes
     unsigned long long *bc = block_clock + (size_t)R3D_NCLOCKS * blockIdx.x;
     bc[0] += C.t_phase[0]; bc[1] += C.t_phase[1]; bc[2] += C.iterations;
     for (int k = 0; k < 4; k++) { bc[3 + k] += C.t_kind[k]; bc[7 + k] += C.n_kind[k]; }
-    bc[11] += C.t_idle;
+    bc[11] += C.t_idle; bc[12] += C.t_collect;
   }
 }
 
