@@ -334,6 +334,56 @@ int r3d_set_snapshots(r3d_handle *h, const r3d_snapshot_desc *s);
  * R3D_EINVAL while snapshots are off. */
 int r3d_fetch_snapshots(r3d_handle *h, double *energy, uint64_t *count, double *outside_energy, uint64_t *outside_count);
 
+/* ---- catch log: which phonons reach chosen seismometers, to be traced again by index ------------------------------------
+ * The bins hold sums; the log keeps the identity of each catch, so that exactly the phonons behind a bin can be traced
+ * again with full event reports (r3d_trace_events_indices).  Draws are keyed by (seed, global phonon index), so a phonon's
+ * index and the run's seed are all a replay needs.
+ *
+ * Log.  While a log is set, every catch that r3d_run bins into a selected seismometer within the bins [bin_lo, bin_hi)
+ * makes one r3d_catch record: all launches of a job, the pilot launches included, with snapshots on or off.  r3d_trace,
+ * r3d_trace_events and the _indices calls make no records.
+ *   - Among the runs of one seed over disjoint index ranges a record is identified uniquely by (phonon, moves, seis).
+ *   - r3d_fetch_catch_log synchronises, concatenates the logs of the handle's devices and returns the kept records sorted
+ *     by (phonon, moves, seis).  A log that is not truncated is therefore independent of scheduling, of how the index
+ *     range was split across calls, and of the devices.
+ *   - *n_matched counts every matching catch.  Each device keeps at most `capacity` records; when *n_matched exceeds the
+ *     records kept, the kept records are an arbitrary subset of the matching catches.
+ *   - Records accumulate across r3d_run calls.  A record does not carry the seed: replay with the seed of its run.
+ *   - r3d_reset empties the log.  r3d_set_catch_log synchronises first and replaces any earlier log (NULL = off).
+ *   - R3D_EINVAL: a seismometer index >= n_seis or listed twice; bin_lo >= bin_hi or bin_hi > n_bins; capacity 0 or above
+ *     R3D_CATCH_LOG_MAX; r3d_fetch_catch_log while the log is off.
+ * The kernels with the log are separate instantiations: with the log off r3d_run runs the same code as without this
+ * feature. */
+#define R3D_CATCH_LOG_MAX (1ull << 28)   /* records per device (16 GB) */
+typedef struct r3d_catch {          /* 64 bytes */
+  uint64_t phonon;                  /* global phonon index                                               */
+  uint32_t seis, bin;               /* seismometer and time bin the catch was added to                    */
+  uint32_t type;                    /* R3D_RAY_P / R3D_RAY_S                                             */
+  uint32_t moves;                   /* move count at the arrival = r3d_event.moves of its COL report      */
+  double   time;                    /* time alive at the arrival (before CatchPhonon's plane-wave shift)  */
+  double   energy[4];               /* X1, X2, X3 and type energy, exactly the addends of the bin         */
+} r3d_catch;
+typedef struct r3d_catch_log_desc {
+  uint32_t n_seis;                  /* entries in seis; 0 = every seismometer       */
+  uint32_t bin_lo, bin_hi;          /* catches into bins [bin_lo, bin_hi)           */
+  uint32_t reserved;
+  const uint32_t *seis;             /* seismometer indices, host memory, borrowed   */
+  uint64_t capacity;                /* records kept per device                      */
+} r3d_catch_log_desc;
+int r3d_set_catch_log(r3d_handle *h, const r3d_catch_log_desc *d);
+/* Writes min(capacity, *n_kept) records to out (out may be NULL when capacity is 0: a query of the two counts).
+ * *n_kept: records kept over all devices; *n_matched: matching catches over all devices. */
+int r3d_fetch_catch_log(r3d_handle *h, r3d_catch *out, uint64_t capacity, uint64_t *n_kept, uint64_t *n_matched);
+
+/* Replay.  r3d_trace / r3d_trace_events for the listed global phonon indices instead of a range, on device slot 0: phonon
+ * indices[i] is traced exactly as r3d_trace(h, indices[i], 1, seed, ...) would trace it.  `indices` must be strictly
+ * increasing (else R3D_EINVAL); an empty list is a no-op.  out[i] of r3d_trace_indices belongs to indices[i]; events are
+ * sorted by (phonon, seq) with r3d_event.phonon the global index.  Bins and counters accumulate as in r3d_trace; no catch
+ * log records are made.  Long lists are split into launches like long ranges. */
+int r3d_trace_indices(r3d_handle *h, const uint64_t *indices, uint64_t n, uint64_t seed, r3d_phonon_final *out);
+int r3d_trace_events_indices(r3d_handle *h, const uint64_t *indices, uint64_t n, uint64_t seed, uint32_t kinds_mask,
+                             r3d_event *out, uint64_t capacity, uint64_t *n_events);
+
 /* Parity hook: trace phonons [first, first+n) on device slot 0 WITHOUT touching
  * the accumulators' semantics (bins are still accumulated) and write each
  * phonon's end state to out[n] (host memory). */

@@ -107,6 +107,32 @@ def snapshot_desc(times, origin, voxel, dims):
     return d, t
 
 
+R3D_CATCH_LOG_MAX = 1 << 28
+
+# struct r3d_catch: one catch-log record
+CATCH_DTYPE = np.dtype([
+    ("phonon", "<u8"), ("seis", "<u4"), ("bin", "<u4"), ("type", "<u4"), ("moves", "<u4"), ("time", "<f8"), ("energy", "<f8", (4,)),
+])
+assert CATCH_DTYPE.itemsize == 64
+
+
+class CatchLogDesc(C.Structure):
+    """struct r3d_catch_log_desc (catch log: seismometers, bin window, records kept per device)"""
+    _fields_ = [("n_seis", C.c_uint32), ("bin_lo", C.c_uint32), ("bin_hi", C.c_uint32), ("reserved", C.c_uint32),
+                ("seis", _pu32), ("capacity", C.c_uint64)]
+
+
+def catch_log_desc(seismometers, bin_lo, bin_hi, capacity):
+    """(CatchLogDesc, the uint32 seismometer array it points into: keep it alive while the descriptor is used).
+    seismometers None = every seismometer."""
+    s = np.ascontiguousarray([] if seismometers is None else seismometers, dtype=np.uint32).reshape(-1)
+    if seismometers is not None and s.size == 0:
+        raise ValueError("an empty seismometer list selects nothing; pass None for every seismometer")
+    d = CatchLogDesc(n_seis=s.size, bin_lo=int(bin_lo), bin_hi=int(bin_hi), seis=as_ptr(s, C.c_uint32) if s.size else None,
+                     capacity=int(capacity))
+    return d, s
+
+
 class ScatterParams(C.Structure):
     """struct r3d_scatter_params (ScatterParams, scatparams.hpp:51-61)"""
     _fields_ = [("nu", C.c_double), ("eps", C.c_double), ("a", C.c_double), ("kappa", C.c_double), ("el", C.c_double), ("gam0", C.c_double)]

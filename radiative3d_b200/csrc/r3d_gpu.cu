@@ -271,6 +271,7 @@ struct JobReq {
   unsigned long long first, n, seed;
   r3d_phonon_final *finals;
   r3d_event *events; unsigned long long *event_cursor, event_cap; uint32_t event_mask;
+  const unsigned long long *replay;        // trace: the device copy of a replayed index list (first = 0, n = its length), or null
 };
 
 struct DevState {
@@ -312,6 +313,9 @@ struct DevState {
   SnapGrid Z{};
   void *snap_mem = nullptr;
   size_t snap_cells = 0;                   // n_times * (n_vox + 1) * 2
+  // catch log (r3d_set_catch_log): G.cap == 0 = off.  The mask, the cursor and the records are one pool allocation, log_mem
+  CatchLog G{};
+  void *log_mem = nullptr;
 };
 
 }  // namespace
@@ -374,19 +378,26 @@ int dev_upload(DevState &D, const T **p, const T *host, size_t count) {
   return 0;
 }
 
-typedef void (*propagate_fn)(const DevModel, const Job, uint32_t, uint32_t, unsigned long long *, unsigned long long *, const SnapGrid);
-// snap: the plain kernel with the energy-snapshot deposits (the trace kernels have none)
-template <class Cell>
-propagate_fn pick_propagate_of(bool trace, bool small, bool snap) {
-  if (snap && !trace) return small ? propagate_kernel<Cell, false, true, true> : propagate_kernel<Cell, false, false, true>;
-  if (small) return trace ? propagate_kernel<Cell, true, true, false> : propagate_kernel<Cell, false, true, false>;
-  return trace ? propagate_kernel<Cell, true, false, false> : propagate_kernel<Cell, false, false, false>;
+typedef void (*propagate_fn)(const DevModel, const Job, uint32_t, uint32_t, unsigned long long *, unsigned long long *, const SnapGrid,
+                             const CatchLog, const unsigned long long *);
+// snap: the plain kernel with the energy-snapshot deposits; log: the plain kernel that writes the catch log (the trace kernels
+// have neither)
+template <class Cell, bool SMALL>
+propagate_fn pick_plain(bool snap, bool log) {
+  if (log) return snap ? propagate_kernel<Cell, false, SMALL, true, true> : propagate_kernel<Cell, false, SMALL, false, true>;
+  return snap ? propagate_kernel<Cell, false, SMALL, true, false> : propagate_kernel<Cell, false, SMALL, false, false>;
 }
-propagate_fn pick_propagate(uint32_t kind, bool trace, bool small, bool wide = false, bool snap = false) {
+template <class Cell>
+propagate_fn pick_propagate_of(bool trace, bool small, bool snap, bool log) {
+  if (trace) return small ? propagate_kernel<Cell, true, true, false, false> : propagate_kernel<Cell, true, false, false, false>;
+  return small ? pick_plain<Cell, true>(snap, log) : pick_plain<Cell, false>(snap, log);
+}
+propagate_fn pick_propagate(uint32_t kind, bool trace, bool small, bool wide = false, bool snap = false, bool log = false) {
   switch (kind) {
-    case R3D_CELL_CYLINDER: return wide ? pick_propagate_of<CylinderWide>(trace, small, snap) : pick_propagate_of<Cylinder>(trace, small, snap);
-    case R3D_CELL_SHELL: return pick_propagate_of<Shell>(trace, small, snap);
-    default: return pick_propagate_of<Tetra>(trace, small, snap);
+    case R3D_CELL_CYLINDER:
+      return wide ? pick_propagate_of<CylinderWide>(trace, small, snap, log) : pick_propagate_of<Cylinder>(trace, small, snap, log);
+    case R3D_CELL_SHELL: return pick_propagate_of<Shell>(trace, small, snap, log);
+    default: return pick_propagate_of<Tetra>(trace, small, snap, log);
   }
 }
 
@@ -672,9 +683,10 @@ int build_device(DevState &D, const r3d_model_desc *d) {
     for (int t = 0; t < 2; t++) D.max_slots[t] = std::max(32u, std::min(D.max_slots[t], (uint32_t)cap / 32 * 32));
   }
   if (D.max_slots[1] < 32) return fail(R3D_EUNSUPPORTED, "shared memory too small for the phonon slots");
-  for (int variant = 0; variant < 3; variant++)          // plain, trace, plain with snapshots
+  for (int variant = 0; variant < 5; variant++)          // plain, trace, plain with snapshots, with the catch log, with both
     for (int wide = 0; wide < (d->cell_kind == R3D_CELL_CYLINDER ? 2 : 1); wide++)
-      CK(cudaFuncSetAttribute(pick_propagate(d->cell_kind, variant == 1, D.table_bytes != 0, wide != 0, variant == 2),
+      CK(cudaFuncSetAttribute(pick_propagate(d->cell_kind, variant == 1, D.table_bytes != 0, wide != 0, variant == 2 || variant == 4,
+                                             variant >= 3),
                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)D.smem_block));
   D.wide_threads = std::min((int)CylinderWide::threads, std::max(32, env_int("R3D_THREADS", CylinderWide::threads) / 32 * 32));
   D.wide = (d->cell_kind == R3D_CELL_CYLINDER) ? env_int("R3D_CYL_WIDE", -1) : 0;      // (-1: decided by the first large job, run_job)
@@ -707,10 +719,12 @@ int run_job(DevState &D, const JobReq &jr) {
   CK(cudaEventRecord(ev0, D.stream));
   const bool trace = jr.finals != nullptr || jr.events != nullptr;
   const bool snap = !trace && D.Z.n_times > 0;        // (also the pilot launches: they trace part of the job)
+  const bool log = !trace && D.G.cap > 0;             // (likewise)
   unsigned long long n_launch = 0;
   auto launch = [&](unsigned long long done, unsigned long long n, bool wide) -> int {
     Job J; J.first = jr.first + done; J.n = n; J.seed = jr.seed; J.finals = jr.finals ? jr.finals + done : nullptr;
     J.events = jr.events; J.event_cursor = jr.event_cursor; J.event_cap = jr.event_cap; J.event_mask = jr.event_mask;
+    const unsigned long long *replay = jr.replay ? jr.replay + done : nullptr;      // (relative index i of this launch = list entry done + i)
     // no more slots than phonons: a small job is spread over all CTAs instead of filling the first few
     uint32_t S = D.max_slots[trace ? 1 : 0];
     const unsigned long long share = (n + (unsigned long long)D.grid - 1) / (unsigned long long)D.grid;
@@ -720,8 +734,8 @@ int run_job(DevState &D, const JobReq &jr) {
     const int grid = (int)std::min<unsigned long long>((unsigned long long)D.grid, need);
     CK(cudaMemsetAsync(D.M.next_phonon, 0, sizeof(unsigned long long), D.stream));
     if (!n_launch) CK(cudaEventRecord(ek0, D.stream));
-    pick_propagate(D.cell_kind, trace, D.table_bytes != 0, wide, snap)<<<grid, wide ? D.wide_threads : D.threads, smem, D.stream>>>(
-        D.M, J, S, D.table_bytes, D.block_tally, D.block_clock, D.Z);
+    pick_propagate(D.cell_kind, trace, D.table_bytes != 0, wide, snap, log)<<<grid, wide ? D.wide_threads : D.threads, smem, D.stream>>>(
+        D.M, J, S, D.table_bytes, D.block_tally, D.block_clock, D.Z, D.G, replay);
     D.launches += 1;
     n_launch++;
     return 0;
@@ -820,11 +834,84 @@ void destroy_device(DevState *D) {
     if (D->stream) cudaStreamSynchronize(D->stream);
     for (void *p : D->allocs) cudaFreeAsync(p, D->stream);
     if (D->snap_mem) cudaFreeAsync(D->snap_mem, D->stream);
+    if (D->log_mem) cudaFreeAsync(D->log_mem, D->stream);
     if (D->stream) cudaStreamSynchronize(D->stream);
     for (int i = 0; i < 7; i++) if (D->ev[i]) cudaEventDestroy(D->ev[i]);
     if (D->stream) cudaStreamDestroy(D->stream);
   }
   delete D;
+}
+
+// The device copy of a list of phonon indices to replay, on the device's stream; freed (stream-ordered) on scope exit.
+struct ReplayList {
+  DevState *D = nullptr;
+  unsigned long long *p = nullptr;
+  int upload(DevState &dev, const uint64_t *idx, uint64_t n) {
+    D = &dev;
+    cudaMemPool_t pool;
+    if (int rc = device_pool(D->device, &pool)) return rc;
+    CK(cudaMallocFromPoolAsync(reinterpret_cast<void **>(&p), n * sizeof(unsigned long long), pool, D->stream));
+    CK(cudaMemcpyAsync(p, idx, n * sizeof(unsigned long long), cudaMemcpyHostToDevice, D->stream));
+    return 0;
+  }
+  ~ReplayList() { if (p) { cudaFreeAsync(p, D->stream); cudaStreamSynchronize(D->stream); } }
+};
+
+int check_indices(const uint64_t *idx, uint64_t n) {
+  if (!idx) return fail(R3D_EINVAL, "null index list");
+  for (uint64_t i = 1; i < n; i++)
+    if (!(idx[i] > idx[i - 1])) return fail(R3D_EINVAL, "replayed phonon indices must be strictly increasing");
+  return 0;
+}
+
+// r3d_trace / r3d_trace_indices: phonons [first, first + n), or (idx != null) the n listed ones
+int trace_finals(r3d_handle *h, uint64_t first_phonon, uint64_t n_phonons, const uint64_t *idx, uint64_t seed, r3d_phonon_final *out) {
+  DevState &D = *h->devs[0];
+  if (int rc = drain(D)) return rc;
+  CK(cudaSetDevice(D.device));
+  ReplayList list;
+  if (idx) { if (int rc = list.upload(D, idx, n_phonons)) return rc; }
+  r3d_phonon_final *dfin = nullptr;
+  CK(cudaMalloc(&dfin, n_phonons * sizeof(r3d_phonon_final)));
+  JobReq jr{}; jr.first = first_phonon; jr.n = n_phonons; jr.seed = seed; jr.finals = dfin; jr.replay = list.p;
+  enqueue(D, jr);
+  int rc = drain(D);
+  cudaError_t e = cudaSuccess;
+  if (!rc) e = cudaMemcpy(out, dfin, n_phonons * sizeof(r3d_phonon_final), cudaMemcpyDeviceToHost);
+  cudaFree(dfin);
+  if (rc) return rc;
+  if (e != cudaSuccess) return fail(R3D_ECUDA, std::string("r3d_trace: ") + cudaGetErrorString(e));
+  return 0;
+}
+
+// r3d_trace_events / r3d_trace_events_indices
+int trace_events(r3d_handle *h, uint64_t first_phonon, uint64_t n_phonons, const uint64_t *idx, uint64_t seed, uint32_t kinds_mask,
+                 r3d_event *out, uint64_t capacity, uint64_t *n_events) {
+  DevState &D = *h->devs[0];
+  if (int rc = drain(D)) return rc;
+  CK(cudaSetDevice(D.device));
+  ReplayList list;
+  if (idx) { if (int rc = list.upload(D, idx, n_phonons)) return rc; }
+  r3d_event *dev = nullptr;
+  unsigned long long *cursor = nullptr;
+  CK(cudaMalloc(&dev, std::max<uint64_t>(capacity, 1) * sizeof(r3d_event)));
+  cudaError_t e = cudaMalloc(&cursor, sizeof(unsigned long long));
+  if (e == cudaSuccess) e = cudaMemset(cursor, 0, sizeof(unsigned long long));
+  if (e != cudaSuccess) { cudaFree(dev); cudaFree(cursor); return fail(R3D_ECUDA, std::string("r3d_trace_events: ") + cudaGetErrorString(e)); }
+  JobReq jr{}; jr.first = first_phonon; jr.n = n_phonons; jr.seed = seed; jr.replay = list.p;
+  jr.events = dev; jr.event_cursor = cursor; jr.event_cap = capacity; jr.event_mask = kinds_mask;
+  enqueue(D, jr);
+  int rc = drain(D);
+  unsigned long long total = 0;
+  if (!rc) e = cudaMemcpy(&total, cursor, sizeof total, cudaMemcpyDeviceToHost);
+  const uint64_t got = std::min<uint64_t>(total, capacity);
+  if (!rc && e == cudaSuccess && got) e = cudaMemcpy(out, dev, got * sizeof(r3d_event), cudaMemcpyDeviceToHost);
+  cudaFree(dev); cudaFree(cursor);
+  if (rc) return rc;
+  if (e != cudaSuccess) return fail(R3D_ECUDA, std::string("r3d_trace_events: ") + cudaGetErrorString(e));
+  std::sort(out, out + got, [](const r3d_event &a, const r3d_event &b) { return a.phonon != b.phonon ? a.phonon < b.phonon : a.seq < b.seq; });
+  *n_events = total;
+  return 0;
 }
 
 }  // namespace
@@ -1013,6 +1100,7 @@ int r3d_reset(r3d_handle *h) {
       CK(cudaMemsetAsync(D.Z.energy, 0, D.snap_cells * sizeof(double), D.stream));
       CK(cudaMemsetAsync(D.Z.count, 0, D.snap_cells * sizeof(unsigned long long), D.stream));
     }
+    if (D.log_mem) CK(cudaMemsetAsync(D.G.cursor, 0, sizeof(unsigned long long), D.stream));      // (records past the cursor are never read)
     CK(cudaStreamSynchronize(D.stream));
   }
   return 0;
@@ -1187,20 +1275,7 @@ int r3d_trace(r3d_handle *h, uint64_t first_phonon, uint64_t n_phonons, uint64_t
   DeviceGuard guard;
   if (!h || !out) return fail(R3D_EINVAL, "null argument");
   if (!n_phonons) return 0;
-  DevState &D = *h->devs[0];
-  if (int rc = drain(D)) return rc;
-  CK(cudaSetDevice(D.device));
-  r3d_phonon_final *dfin = nullptr;
-  CK(cudaMalloc(&dfin, n_phonons * sizeof(r3d_phonon_final)));
-  JobReq jr{}; jr.first = first_phonon; jr.n = n_phonons; jr.seed = seed; jr.finals = dfin;
-  enqueue(D, jr);
-  int rc = drain(D);
-  cudaError_t e = cudaSuccess;
-  if (!rc) e = cudaMemcpy(out, dfin, n_phonons * sizeof(r3d_phonon_final), cudaMemcpyDeviceToHost);
-  cudaFree(dfin);
-  if (rc) return rc;
-  if (e != cudaSuccess) return fail(R3D_ECUDA, std::string("r3d_trace: ") + cudaGetErrorString(e));
-  return 0;
+  return trace_finals(h, first_phonon, n_phonons, nullptr, seed, out);
 }
 
 int r3d_trace_events(r3d_handle *h, uint64_t first_phonon, uint64_t n_phonons, uint64_t seed, uint32_t kinds_mask,
@@ -1209,28 +1284,107 @@ int r3d_trace_events(r3d_handle *h, uint64_t first_phonon, uint64_t n_phonons, u
   if (!h || !n_events || (capacity && !out)) return fail(R3D_EINVAL, "null argument");
   *n_events = 0;
   if (!n_phonons) return 0;
-  DevState &D = *h->devs[0];
-  if (int rc = drain(D)) return rc;
-  CK(cudaSetDevice(D.device));
-  r3d_event *dev = nullptr;
-  unsigned long long *cursor = nullptr;
-  CK(cudaMalloc(&dev, std::max<uint64_t>(capacity, 1) * sizeof(r3d_event)));
-  cudaError_t e = cudaMalloc(&cursor, sizeof(unsigned long long));
-  if (e == cudaSuccess) e = cudaMemset(cursor, 0, sizeof(unsigned long long));
-  if (e != cudaSuccess) { cudaFree(dev); cudaFree(cursor); return fail(R3D_ECUDA, std::string("r3d_trace_events: ") + cudaGetErrorString(e)); }
-  JobReq jr{}; jr.first = first_phonon; jr.n = n_phonons; jr.seed = seed;
-  jr.events = dev; jr.event_cursor = cursor; jr.event_cap = capacity; jr.event_mask = kinds_mask;
-  enqueue(D, jr);
-  int rc = drain(D);
-  unsigned long long total = 0;
-  if (!rc) e = cudaMemcpy(&total, cursor, sizeof total, cudaMemcpyDeviceToHost);
-  const uint64_t got = std::min<uint64_t>(total, capacity);
-  if (!rc && e == cudaSuccess && got) e = cudaMemcpy(out, dev, got * sizeof(r3d_event), cudaMemcpyDeviceToHost);
-  cudaFree(dev); cudaFree(cursor);
-  if (rc) return rc;
-  if (e != cudaSuccess) return fail(R3D_ECUDA, std::string("r3d_trace_events: ") + cudaGetErrorString(e));
-  std::sort(out, out + got, [](const r3d_event &a, const r3d_event &b) { return a.phonon != b.phonon ? a.phonon < b.phonon : a.seq < b.seq; });
-  *n_events = total;
+  return trace_events(h, first_phonon, n_phonons, nullptr, seed, kinds_mask, out, capacity, n_events);
+}
+
+int r3d_trace_indices(r3d_handle *h, const uint64_t *indices, uint64_t n, uint64_t seed, r3d_phonon_final *out) {
+  DeviceGuard guard;
+  if (!h || (n && !out)) return fail(R3D_EINVAL, "null argument");
+  if (!n) return 0;
+  if (int rc = check_indices(indices, n)) return rc;
+  return trace_finals(h, 0, n, indices, seed, out);
+}
+
+int r3d_trace_events_indices(r3d_handle *h, const uint64_t *indices, uint64_t n, uint64_t seed, uint32_t kinds_mask,
+                             r3d_event *out, uint64_t capacity, uint64_t *n_events) {
+  DeviceGuard guard;
+  if (!h || !n_events || (capacity && !out)) return fail(R3D_EINVAL, "null argument");
+  *n_events = 0;
+  if (!n) return 0;
+  if (int rc = check_indices(indices, n)) return rc;
+  return trace_events(h, 0, n, indices, seed, kinds_mask, out, capacity, n_events);
+}
+
+int r3d_set_catch_log(r3d_handle *h, const r3d_catch_log_desc *d) {
+  DeviceGuard guard;
+  if (!h) return fail(R3D_EINVAL, "null handle");
+  const size_t words = std::max<size_t>(1, ((size_t)h->n_seis + 31) / 32);
+  std::vector<uint32_t> mask(words, 0u);
+  if (d) {
+    if (d->n_seis && !d->seis) return fail(R3D_EINVAL, "null seismometer list");
+    for (uint32_t i = 0; i < (d->n_seis ? d->n_seis : h->n_seis); i++) {
+      const uint32_t k = d->n_seis ? d->seis[i] : i;
+      if (k >= h->n_seis) return fail(R3D_EINVAL, "catch log: seismometer index out of range");
+      if ((mask[k >> 5] >> (k & 31u)) & 1u) return fail(R3D_EINVAL, "catch log: seismometer listed twice");
+      mask[k >> 5] |= 1u << (k & 31u);
+    }
+    if (d->bin_lo >= d->bin_hi || d->bin_hi > h->n_bins) return fail(R3D_EINVAL, "catch log: need bin_lo < bin_hi <= n_bins");
+    if (!d->capacity || d->capacity > R3D_CATCH_LOG_MAX) return fail(R3D_EINVAL, "catch log: capacity must be in [1, R3D_CATCH_LOG_MAX]");
+  }
+  for (DevState *Dp : h->devs) {
+    DevState &D = *Dp;
+    if (int rc = drain(D)) return rc;
+    CK(cudaSetDevice(D.device));
+    CK(cudaStreamSynchronize(D.stream));
+    if (D.log_mem) CK(cudaFreeAsync(D.log_mem, D.stream));
+    D.log_mem = nullptr;
+    D.G = CatchLog{};
+    if (!d) continue;
+    // [capacity] records | cursor | mask words
+    cudaMemPool_t pool;
+    if (int rc = device_pool(D.device, &pool)) return rc;
+    CK(cudaMallocFromPoolAsync(&D.log_mem, d->capacity * sizeof(r3d_catch) + sizeof(unsigned long long) + words * sizeof(uint32_t), pool,
+                               D.stream));
+    D.G.rec = static_cast<r3d_catch *>(D.log_mem);
+    D.G.cursor = reinterpret_cast<unsigned long long *>(D.G.rec + d->capacity);
+    uint32_t *m = reinterpret_cast<uint32_t *>(D.G.cursor + 1);
+    D.G.mask = m;
+    CK(cudaMemsetAsync(D.G.cursor, 0, sizeof(unsigned long long), D.stream));
+    CK(cudaMemcpyAsync(m, mask.data(), words * sizeof(uint32_t), cudaMemcpyHostToDevice, D.stream));
+    D.G.cap = d->capacity; D.G.bin_lo = d->bin_lo; D.G.bin_hi = d->bin_hi;
+    CK(cudaStreamSynchronize(D.stream));                     // (mask goes out of scope)
+  }
+  return 0;
+}
+
+int r3d_fetch_catch_log(r3d_handle *h, r3d_catch *out, uint64_t capacity, uint64_t *n_kept, uint64_t *n_matched) {
+  DeviceGuard guard;
+  if (!h) return fail(R3D_EINVAL, "null handle");
+  if (capacity && !out) return fail(R3D_EINVAL, "null output array");
+  if (h->devs.empty() || !h->devs[0]->log_mem) return fail(R3D_EINVAL, "the catch log is off (r3d_set_catch_log)");
+  const size_t G = h->devs.size();
+  std::vector<unsigned long long> cur(G, 0);
+  uint64_t matched = 0, kept = 0;
+  for (size_t g = 0; g < G; g++) {
+    DevState &D = *h->devs[g];
+    if (int rc = drain(D)) return rc;
+    CK(cudaSetDevice(D.device));
+    CK(cudaMemcpyAsync(&cur[g], D.G.cursor, sizeof(unsigned long long), cudaMemcpyDeviceToHost, D.stream));
+    CK(cudaStreamSynchronize(D.stream));
+    matched += cur[g];
+    kept += std::min<unsigned long long>(cur[g], D.G.cap);
+  }
+  if (capacity && kept) {
+    // every device's kept records, in device order, then sorted: directly in `out` when it holds them all
+    std::vector<r3d_catch> tmp;
+    r3d_catch *all = out;
+    if (capacity < kept) { tmp.resize(kept); all = tmp.data(); }
+    uint64_t at = 0;
+    for (size_t g = 0; g < G; g++) {
+      DevState &D = *h->devs[g];
+      const uint64_t k = std::min<unsigned long long>(cur[g], D.G.cap);
+      CK(cudaSetDevice(D.device));
+      if (k) CK(cudaMemcpyAsync(all + at, D.G.rec, k * sizeof(r3d_catch), cudaMemcpyDeviceToHost, D.stream));
+      CK(cudaStreamSynchronize(D.stream));
+      at += k;
+    }
+    std::sort(all, all + kept, [](const r3d_catch &a, const r3d_catch &b) {
+      return a.phonon != b.phonon ? a.phonon < b.phonon : a.moves != b.moves ? a.moves < b.moves : a.seis < b.seis;
+    });
+    if (all != out) memcpy(out, all, capacity * sizeof(r3d_catch));
+  }
+  if (n_kept) *n_kept = kept;
+  if (n_matched) *n_matched = matched;
   return 0;
 }
 

@@ -79,6 +79,17 @@ struct SnapGrid {
   double origin[3], voxel[3];
   uint32_t dims[3], n_vox, n_times;
 };
+// ---- catch log (include/r3d_gpu.h r3d_set_catch_log) ----------------------------------------------------------------------
+// The log of one device: every catch into a selected seismometer and bin window takes the next record (one atomic on the
+// cursor per warp pass with records).  A kernel parameter after the snapshot grid, like it, so that the kernels without the
+// log keep their parameter layout.
+struct CatchLog {
+  const uint32_t *mask;             // bit k % 32 of word k / 32: seismometer k is selected
+  r3d_catch *rec;                   // [cap]
+  unsigned long long *cursor;       // matching catches so far; records [0, min(cursor, cap)) are written
+  unsigned long long cap;
+  uint32_t bin_lo, bin_hi;          // bins [bin_lo, bin_hi)
+};
 // One move, as a deposit needs it: everything is what the phonon had in registers when it moved (the move's Path is
 // derived again from the start point, by the same function, only for moves that straddle a snapshot time).
 struct SnapMove {
@@ -138,8 +149,20 @@ struct Tally {
 #define R3D_SLOT_BYTES_TRACE 154u      // + FP64 path length / recent travel time (8) + four u32 per-phonon counters (16)
 extern __shared__ __align__(16) unsigned char r3d_smem[];
 struct Clock4 { double time, pathlen, recent, aexp; };
+// The global phonon index of a slot's relative index `rel`: the job's first index + rel, or - trace kernels replaying a list
+// (r3d_trace_indices) - entry rel of the list.  An empty base of Slots without the list, so that the plain kernels' Slots
+// stays what it was (a member, even unused, changed their code).
+template <bool TRACE> struct SlotIndex {
+  R3D_DEV void set_replay(const unsigned long long *) {}
+  R3D_DEV unsigned long long index_of(const Job &J, unsigned long long rel) const { return J.first + rel; }
+};
+template <> struct SlotIndex<true> {
+  const unsigned long long *replay;  // [relative index] -> global index, or null
+  R3D_DEV void set_replay(const unsigned long long *r) { replay = r; }
+  R3D_DEV unsigned long long index_of(const Job &J, unsigned long long rel) const { return replay ? __ldg(replay + rel) : J.first + rel; }
+};
 template <bool TRACE>
-struct Slots {
+struct Slots : SlotIndex<TRACE> {
   uint32_t S, table_bytes;      // table_bytes: the staged small-model tables (multiple of 16; 0 = none)
   static constexpr uint32_t kState = TRACE ? R3D_SLOT_STATE_TRACE : R3D_SLOT_STATE;
   R3D_DEV double &time(uint32_t s) const { return reinterpret_cast<double *>(r3d_smem)[s]; }                        // time alive
@@ -342,7 +365,7 @@ R3D_DEV void emit(const Slots<TRACE> &A, const Job &J, uint32_t s, uint32_t kind
   const unsigned long long at = atomicAdd(J.event_cursor, 1ull);
   if (at >= J.event_cap) return;
   r3d_event *e = J.events + at;
-  e->phonon = J.first + A.idx(s); e->seq = seq; e->kind = kind; e->type = (uint32_t)type; e->moves = moves; e->cell = cell; e->reason = reason;
+  e->phonon = A.index_of(J, A.idx(s)); e->seq = seq; e->kind = kind; e->type = (uint32_t)type; e->moves = moves; e->cell = cell; e->reason = reason;
   e->time = time; e->pathlen = pathlen; e->loc[0] = loc.x; e->loc[1] = loc.y; e->loc[2] = loc.z;
   angles_of(dir, e->theta, e->phi);
   e->amp = exp(-aexp);
@@ -499,7 +522,7 @@ R3D_DEV int advance_one(const DevModel &M, const Job &J, const Slots<TRACE> &A, 
     // taking it before keeps the generator's state and the logarithm out of the registers while the ray geometry - up to 20
     // doubles of scratch for a curved ray - is live.  A phonon that times out on an infinite path has consumed no draw:
     // `ordinal` only moves further down.)
-    Rng g; g.init(J.seed, J.first + A.idx(s));
+    Rng g; g.init(J.seed, A.index_of(J, A.idx(s)));
     const uint32_t o = ordinal & 3u, b = ordinal >> 2;
     g.block(b);
     const uint32_t w1 = g.w[1], w2 = g.w[2], w3 = g.w[3];
@@ -606,7 +629,7 @@ R3D_DEV int advance_one(const DevModel &M, const Job &J, const Slots<TRACE> &A, 
 // PhononSource::GenerateRandomPhonon (sources.cpp:156-170) -> Phonon ctor (phonons.hpp:193-207)
 template <bool TRACE>
 R3D_DEV void refill_one(const DevModel &M, const Job &J, const Slots<TRACE> &A, uint32_t s, unsigned long long rel, Tally &T) {
-  const unsigned long long idx = J.first + rel;
+  const unsigned long long idx = A.index_of(J, rel);
   Rng g; g.init(J.seed, idx);
   g.block(0);
   const uint32_t rt3 = cdf_search_small(M.src_whole, 3, g.w[0] >> 1);
@@ -776,9 +799,54 @@ R3D_DEV void draw_batch(const DevModel &M, const Job &J, const Slots<TRACE> &A, 
 // the L1-to-L2 write throughput, profiles/r2_histogram.md), so there is nothing for an aggregation step in shared memory
 // to win; catches per (seismometer, bin) are independent arrivals.
 // All 32 lanes call this; `have` = the lane holds a slot of the chunk.
+// LOG kernels also record every selected catch of a pass in the catch log G (log_catches); the others get G = null.
 // =====================================================================================================
-template <class Cell, bool TRACE, class TabT>
-R3D_DEV void collect_warp(const DevModel &M, const Slots<TRACE> &A, const TabT &tab, bool have, uint32_t s, Tally &T) {
+// The catch-log records of one warp pass of collect_warp: one ballot, one atomic on the cursor for the pass's records, each
+// lane writes its record at its rank (when that is below the capacity).  All 32 lanes call this.
+template <bool TRACE>
+R3D_DEV void log_catches(const Slots<TRACE> &A, const Job &J, const CatchLog &G, bool logged, uint32_t s, uint32_t seis, uint32_t bin,
+                         const double (&e)[4]) {
+  const unsigned b = __ballot_sync(R3D_FULL, logged);
+  if (!b) return;
+  const unsigned lane = threadIdx.x & 31u;
+  const int leader = __ffs(b) - 1;
+  unsigned long long at = 0;
+  if ((int)lane == leader) at = atomicAdd(G.cursor, (unsigned long long)__popc(b));
+  at = __shfl_sync(R3D_FULL, at, leader) + (unsigned long long)__popc(b & ((1u << lane) - 1u));
+  if (!logged || at >= G.cap) return;
+  const uint4 meta = A.meta(s);
+  ulonglong2 *o = reinterpret_cast<ulonglong2 *>(G.rec + at);          // r3d_catch, 64 bytes: four 16-byte stores
+  o[0] = make_ulonglong2(J.first + A.idx(s), (unsigned long long)seis | ((unsigned long long)bin << 32));
+  o[1] = make_ulonglong2((unsigned long long)meta.w | ((unsigned long long)meta.x << 32), (unsigned long long)__double_as_longlong(A.time(s)));
+  reinterpret_cast<double2 *>(o)[2] = make_double2(e[0], e[1]);
+  reinterpret_cast<double2 *>(o)[3] = make_double2(e[2], e[3]);
+}
+
+// A lane's catch-log record in the making.  Without the log it has no state and no code (so that the kernels without the log
+// compile exactly as they did before it existed: dead locals in the pass loop were enough to change their register allocation).
+template <bool LOG> struct LaneCatch {
+  R3D_DEV void select(const CatchLog *, uint32_t, uint32_t, const double (&)[4]) {}
+  template <bool TRACE> R3D_DEV void write(const Slots<TRACE> &, const Job &, const CatchLog *, uint32_t) {}
+};
+template <> struct LaneCatch<true> {
+  bool logged = false;
+  uint32_t seis = 0, bin = 0;
+  double e[4] = {0.0, 0.0, 0.0, 0.0};
+  // after a successful seis_catch: keep the catch if its seismometer and bin are selected
+  R3D_DEV void select(const CatchLog *G, uint32_t k, uint32_t b, const double (&x)[4]) {
+    if (b >= G->bin_lo && b < G->bin_hi && ((__ldg(G->mask + (k >> 5)) >> (k & 31u)) & 1u)) {
+      logged = true; seis = k; bin = b;
+      e[0] = x[0]; e[1] = x[1]; e[2] = x[2]; e[3] = x[3];
+    }
+  }
+  template <bool TRACE> R3D_DEV void write(const Slots<TRACE> &A, const Job &J, const CatchLog *G, uint32_t s) {
+    log_catches<TRACE>(A, J, *G, logged, s, seis, bin, e);
+  }
+};
+
+template <class Cell, bool TRACE, bool LOG, class TabT>
+R3D_DEV void collect_warp(const DevModel &M, const Job &J, const Slots<TRACE> &A, const TabT &tab, bool have, uint32_t s, Tally &T,
+                          const CatchLog *G) {
   if (M.n_seis == 0) return;
   const unsigned lane = threadIdx.x & 31u;
   uint32_t i0 = 0, i1 = 0;
@@ -817,6 +885,7 @@ R3D_DEV void collect_warp(const DevModel &M, const Slots<TRACE> &A, const TabT &
       if (__shfl_sync(R3D_FULL, end, owner + step - 1u) <= p) owner += step;
     }
     const uint32_t ss = __shfl_sync(R3D_FULL, s, owner), j = __shfl_sync(R3D_FULL, off, owner) + p;
+    LaneCatch<LOG> lc;                                  // LOG: this pair's catch, when the catch log selects it
     if (p < total) {
       const uint32_t k2 = __ldg(M.grid_items + j);
       const double2 qa = __ldg(reinterpret_cast<const double2 *>(M.seis_sphere + k2));
@@ -843,9 +912,11 @@ R3D_DEV void collect_warp(const DevModel &M, const Slots<TRACE> &A, const TabT &
           atomicAdd(M.counts + bb * 2 + type, 1ull);
           caught++;
           if (TRACE) atomicAdd(&A.tr(0, ss), 1u);                 // catches are rare: one shared atomic each
+          lc.select(G, k2, bin, e);
         }
       }
     }
+    lc.write(A, J, G, ss);                              // (the warp is converged here)
   }
   T.v[R3D_CNT_CATCHES] += caught;                      // (a tally is summed over the threads at the end: whose it is does not matter)
 }
@@ -987,13 +1058,16 @@ R3D_DEV void snap_deposit(const DevModel &M, const SnapGrid &Z, const TabT &tab,
 // =====================================================================================================
 // the kernel: persistent CTAs, S slots each
 // =====================================================================================================
-template <class Cell, bool TRACE, bool SMALL, bool SNAP>
+// LOG: the catch log (plain kernels only); `replay`: the list a trace kernel replays (r3d_trace_indices), or null.  G and
+// replay come after all other parameters, so that adding them left the others' layout as it was.
+template <class Cell, bool TRACE, bool SMALL, bool SNAP, bool LOG>
 __global__ void __launch_bounds__(Cell::threads, 1)
 propagate_kernel(const DevModel M, const Job J, uint32_t S, uint32_t table_bytes, unsigned long long *block_tally,
-                 unsigned long long *block_clock, const SnapGrid Z) {
+                 unsigned long long *block_clock, const SnapGrid Z, const CatchLog G, const unsigned long long *replay) {
+  static_assert(!(TRACE && LOG), "the trace kernels make no catch-log records");
   __shared__ unsigned long long tally_sm[R3D_NT / 32][R3D_NCOUNTERS];
   __shared__ Ctl C;
-  Slots<TRACE> A; A.S = S; A.table_bytes = table_bytes;
+  Slots<TRACE> A; A.S = S; A.table_bytes = table_bytes; A.set_replay(replay);
   Tab<SMALL> tab; tab.init(M, S * Slots<TRACE>::kState);
   tab.stage(M);
   log_table_fill(log_table());
@@ -1114,7 +1188,7 @@ propagate_kernel(const DevModel M, const Job J, uint32_t S, uint32_t table_bytes
 #if R3D_CHUNK_CLOCKS
           const long long tcc = clock64();
 #endif
-          collect_warp<Cell, TRACE>(M, A, tab, have, s, T);
+          collect_warp<Cell, TRACE, LOG>(M, J, A, tab, have, s, T, LOG ? &G : nullptr);     // (G by reference changed the plain kernels' code)
 #if R3D_CHUNK_CLOCKS
           if (lane == 0) atomicAdd(&C.t_collect, (unsigned long long)(clock64() - tcc));
 #endif

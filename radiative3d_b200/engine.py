@@ -10,6 +10,7 @@ the calls raise.  Nothing in this module imports or executes anything under orac
 """
 import ctypes as C
 import os
+import warnings
 
 import numpy as np
 
@@ -23,6 +24,7 @@ EXPORTS = [
     "r3d_create", "r3d_run", "r3d_sync", "r3d_fetch", "r3d_reset", "r3d_device_accumulators", "r3d_device_accumulator_blocks", "r3d_stream",
     "r3d_launch_count", "r3d_trace", "r3d_trace_events", "r3d_build_scatterer_tables", "r3d_toa_create", "r3d_scatterer_g_values", "r3d_toa_destroy", "r3d_set_profiling", "r3d_kernel_times", "r3d_test_cdf_search", "r3d_test_path_to_boundary", "r3d_test_advance",
     "r3d_test_advance_time", "r3d_set_snapshots", "r3d_fetch_snapshots", "r3d_test_transform", "r3d_test_rtcoef", "r3d_test_catch", "r3d_test_arith", "r3d_test_pathlog", "r3d_destroy", "r3d_last_error", "r3d_abi_version",
+    "r3d_set_catch_log", "r3d_fetch_catch_log", "r3d_trace_indices", "r3d_trace_events_indices",
 ]
 
 
@@ -57,6 +59,10 @@ def load_library(path=None):
     L.r3d_launch_count.argtypes = [vp, pu64]
     L.r3d_trace.argtypes = [vp, C.c_uint64, C.c_uint64, C.c_uint64, vp]
     L.r3d_trace_events.argtypes = [vp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32, vp, C.c_uint64, pu64]
+    L.r3d_trace_indices.argtypes = [vp, vp, C.c_uint64, C.c_uint64, vp]
+    L.r3d_trace_events_indices.argtypes = [vp, vp, C.c_uint64, C.c_uint64, C.c_uint32, vp, C.c_uint64, pu64]
+    L.r3d_set_catch_log.argtypes = [vp, C.POINTER(abi.CatchLogDesc)]
+    L.r3d_fetch_catch_log.argtypes = [vp, vp, C.c_uint64, pu64, pu64]
     L.r3d_build_scatterer_tables.argtypes = [C.POINTER(abi.ScatterParams), C.c_uint32, pd, pd, C.c_uint32, C.c_int, pd, pd, pd, pd]
     L.r3d_set_profiling.argtypes = [vp, C.c_int]
     L.r3d_kernel_times.argtypes = [vp, pd, pu64, pu64]
@@ -185,6 +191,50 @@ class Engine:
         _ck(self._L, self._L.r3d_trace_events(self._h, first_phonon, n_phonons, seed, kinds, out.ctypes.data, cap, C.byref(n)))
         if n.value > cap:
             raise R3DError(abi.R3D_EINVAL if hasattr(abi, "R3D_EINVAL") else 1, f"{n.value} events occurred, room for {cap}")
+        return out[:n.value]
+
+    # -- catch log and replay by index (include/r3d_gpu.h r3d_set_catch_log) --
+    def set_catch_log(self, seismometers=None, bins=None, capacity=1 << 24):
+        """Log every catch of the following runs into the seismometers `seismometers` (indices; None = all) within the bins
+        `bins` = (lo, hi), [lo, hi) (None = all), keeping at most `capacity` records per device; an empty log.
+        `capacity` None turns the log off."""
+        if capacity is None:
+            _ck(self._L, self._L.r3d_set_catch_log(self._h, None))
+            return
+        lo, hi = (0, self.model.n_bins) if bins is None else bins
+        d, keep = abi.catch_log_desc(seismometers, lo, hi, capacity)
+        _ck(self._L, self._L.r3d_set_catch_log(self._h, C.byref(d)))
+        del keep
+
+    def fetch_catch_log(self):
+        """(records, n_matched): the kept catch-log records (abi.CATCH_DTYPE) of all devices sorted by (phonon, moves, seis),
+        and the number of matching catches.  Warns when records were dropped (n_matched > len(records))."""
+        kept, matched = C.c_uint64(), C.c_uint64()
+        _ck(self._L, self._L.r3d_fetch_catch_log(self._h, None, 0, C.byref(kept), C.byref(matched)))
+        out = np.zeros(kept.value, dtype=abi.CATCH_DTYPE)
+        if kept.value:
+            _ck(self._L, self._L.r3d_fetch_catch_log(self._h, out.ctypes.data, kept.value, C.byref(kept), C.byref(matched)))
+        if matched.value > out.size:
+            warnings.warn(f"catch log: {matched.value} catches matched, {out.size} records kept (capacity per device too small)",
+                          RuntimeWarning, stacklevel=2)
+        return out, int(matched.value)
+
+    def trace_indices(self, indices, seed=20261018):
+        """trace() for the listed global phonon indices (strictly increasing): out[i] belongs to indices[i]."""
+        idx = np.ascontiguousarray(indices, dtype=np.uint64).reshape(-1)
+        out = np.zeros(idx.size, dtype=abi.PHONON_FINAL_DTYPE)
+        _ck(self._L, self._L.r3d_trace_indices(self._h, idx.ctypes.data, idx.size, seed, out.ctypes.data))
+        return out
+
+    def trace_events_indices(self, indices, seed=20261018, kinds=abi.R3D_EV_ALL, capacity=None):
+        """trace_events() for the listed global phonon indices (strictly increasing), sorted by (phonon, seq)."""
+        idx = np.ascontiguousarray(indices, dtype=np.uint64).reshape(-1)
+        cap = int(capacity or max(4096, 512 * idx.size))
+        out = np.zeros(cap, dtype=abi.EVENT_DTYPE)
+        n = C.c_uint64()
+        _ck(self._L, self._L.r3d_trace_events_indices(self._h, idx.ctypes.data, idx.size, seed, kinds, out.ctypes.data, cap, C.byref(n)))
+        if n.value > cap:
+            raise R3DError(abi.R3D_EINVAL, f"{n.value} events occurred, room for {cap}")
         return out[:n.value]
 
     # -- energy snapshots (include/r3d_gpu.h r3d_set_snapshots) --
