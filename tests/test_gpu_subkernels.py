@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 import oracle_binding as ob
+import seis_layouts
 from conftest import CONFIGS, GOLDEN, load_golden, rel_err
 from radiative3d_b200 import abi, engine
 
@@ -154,6 +155,15 @@ def test_catch(cfg):
     assert np.array_equal(out[:, :2], ref[:, :2])
     assert np.array_equal(out[:, :2], z["catch_out"][:, :2])
     assert rel_err(out[:, 2:], ref[:, 2:]).max() <= TOL
+    # the annulus branch (r_in > 0, no shift), which no golden station has, and the radius and bin edges
+    rows, want = seis_layouts.catch_edge_rows(m, z["catch_in"])
+    out = engine.catch(m.bin_dt, m.n_bins, rows)
+    ref = ob.catch(m.bin_dt, m.n_bins, rows)
+    assert np.array_equal(out[:, :2], ref[:, :2])
+    edge = want >= 0
+    assert np.array_equal(out[edge, 0], want[edge])
+    assert np.array_equal(out[:, 5], ref[:, 5])
+    assert rel_err(out[:, 2:5], ref[:, 2:5]).max() <= TOL
 
 
 def test_branch_free_arithmetic():
